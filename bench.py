@@ -2,6 +2,7 @@
 """bench.py — throughput of the MRI artifact chain on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg3|cfg1]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic volumes (SURVEY.md 8(d)):
   cfg2 (default, the configuration BASELINE.json's metric is quoted on): the 127-series chain
@@ -14,6 +15,9 @@ metric through the public API with HOST buffers (pinned H2D of the inputs and D2
 inside the timed region); `roofline` = dominant kernel against the measured HBM peak;
 `cpu_baseline` = the oracle port of the reference timed on this box's host cores.
 With --impl reference only the CPU reference arm runs (rank 0), on the same config and metric.
+--dump-outputs DIR writes what the last timed step returned on rank 0 as DIR/out.npy (see output_sample), so that
+two builds can be compared output for output: the inputs, spike locations and S&P seeds are fixed, so the same
+arguments give the same inputs on every run.
 """
 import argparse
 import json
@@ -56,6 +60,28 @@ WORKLOADS = {
 }
 # configs[3] and configs[4] of BASELINE.json have other units of work (2-D slices; 128x128x64 crops): bench.py --workload cfg4|cfg5
 AUX_WORKLOADS = ("cfg4", "cfg5", "train127")
+DUMP_BYTES = 32 << 20          # --dump-outputs: largest array written whole; larger outputs are sampled down to it
+
+
+def output_sample(y, budget=DUMP_BYTES):
+    """y as a float32 (float64 if it is one) host array: whole if it fits in `budget` bytes, else at most the k elements
+    that fit, taken from y.reshape(-1) at increasing positions whose gaps numpy.random.default_rng(0) draws uniformly
+    from [1, 2 n / k) (n elements): the same positions for the same output shape on every run."""
+    y = torch.as_tensor(y).detach()
+    if y.dtype != torch.float64:
+        y = y.to(torch.float32)
+    n, k = y.numel(), budget // y.element_size()
+    if n <= k:
+        return y.cpu().numpy()
+    idx = np.cumsum(np.random.default_rng(0).integers(1, 2 * (n // k), size=k)) - 1
+    idx = idx[idx < n]
+    return y.reshape(-1)[torch.from_numpy(idx).to(y.device)].cpu().numpy()
+
+
+def write_outputs(dirname, arrays):
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def peak_hbm():
@@ -366,11 +392,13 @@ def run_aux_workload(args):
             flush.zero_()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            step()
+            y = step()
             b.record()
             torch.cuda.synchronize(dev)
             tot += a.elapsed_time(b)
         launches = int(L.mvtb_launch_count() - n0)
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, {"out": output_sample(y)})
     stats = torch.tensor([tot, float(units)], dtype=torch.float64, device=dev)
     mx, sm = aggregate(stats, world)
     if rank == 0:
@@ -401,7 +429,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer leg (kernel sweeps)")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle spot check printed in the JSON line")
     ap.add_argument("--disk-r", type=float, default=None, help="override the disk radius (sweeps; the headline uses the workload's 12.5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step (rank 0) to DIR/out.npy, sampled down to %d MB if larger"
+                         % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.workload in AUX_WORKLOADS:
         return run_aux_workload(args)
     cfg = dict(WORKLOADS[args.workload])
@@ -460,7 +495,7 @@ def main():
     th0 = time.perf_counter()
     e0.record()
     for s in range(args.steps):
-        gpu_step(cfg, x, idxs, out, 100 + s)
+        y = gpu_step(cfg, x, idxs, out, 100 + s)
     e1.record()
     barrier()
     th1 = time.perf_counter()
@@ -468,6 +503,8 @@ def main():
     launches = int(L.mvtb_launch_count() - launches0)
     clocks = sampler.stop(th0, th1)
     checksum = float(out.double().sum())
+    # taken before the profiling and parity passes below reuse `out`
+    dumped = {"out": output_sample(y)} if args.dump_outputs and rank == 0 else None
 
     # ---- per-kernel device time (cudaEvents around every launch, on the launching stream)
     plan = Fn.get_plan(SHAPE, vols_per_step, dev)
@@ -625,6 +662,8 @@ def main():
     ms, e2e_ms, ceiling_ms = float(mx[0]), float(mx[1]), float(mx[4])
     total_vols_per_step, checksum, total_e2e_per_step = float(sm[2]), float(sm[3]), float(sm[5])
 
+    if dumped:
+        write_outputs(args.dump_outputs, dumped)
     if rank == 0:
         value = total_vols_per_step * args.steps / (ms * 1e-3)
         e2e_value = total_e2e_per_step * e2e_steps / (e2e_ms * 1e-3) if e2e_steps else None

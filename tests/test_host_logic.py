@@ -285,6 +285,28 @@ def test_bench_reference_arm_json_contract():
     assert cb["kind"] in ("reference", "port") and cb["value_1_thread"] > 0 and cb["cores"] >= 1 and cb["value"] == line["value"] and cb["sample"]
 
 
+def test_bench_output_sample_is_whole_or_a_fixed_sample():
+    """`bench.py --dump-outputs`: an output that fits is written whole; a larger one is sampled at the same positions
+    on every run, in float32 (float64 stays float64)."""
+    import bench
+    y = torch.arange(1000, dtype=torch.float32).reshape(10, 100)
+    assert np.array_equal(bench.output_sample(y, budget=4000), y.numpy())
+    a = bench.output_sample(y, budget=400)
+    assert a.dtype == np.float32 and 50 < a.size <= 100 and np.all(np.diff(a) > 0)       # sorted distinct positions
+    assert np.array_equal(a, bench.output_sample(y.clone(), budget=400))
+    d = bench.output_sample(y.double(), budget=800)                                          # same element count
+    assert d.dtype == np.float64 and np.array_equal(d, a)
+    assert bench.output_sample(y.to(torch.float16), budget=4000).dtype == np.float32
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_rejects_arguments_it_cannot_honour(argv):
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 2 and "error:" in out.stderr and not out.stdout
+
+
 def test_gibbs_layer_reads_alpha_once_per_update():
     """GibbsNoiseLayer keeps alpha's host value until the attribute is reassigned or written in place (S:71 reads it
     on the host every forward; on a CUDA tensor that is a synchronising copy)."""
