@@ -201,6 +201,34 @@ int mvtb_crop_flip_f32(const float* in, float* out, int n_channels, const int32_
 int mvtb_crop_flip_batch_f32(const float* in, float* out, int n_samples, int n_channels, const int32_t* in_shape,
                              const int32_t* out_shape, const int32_t* offsets_dev, const int32_t* flips_dev, void* stream);
 
+/* Spacingd -> Orientationd (MONAI 0.5, 127_...FLAIR.py:120-129: pixdim (1.5, 1.5, 2.0), modes bilinear / nearest,
+ * border padding, align_corners=False; then axcodes "RAS"), optionally followed by a crop and flip, as one gather from
+ * the loaded volume.  in: (n_volumes, H, W, D), out: (n_volumes, s0, s1, s2), contiguous fp32, in != out.
+ * Output index j -> index q in Spacingd's output grid:  q[g] = base[g] + step[g] * j[axis[g]]  (axis a permutation,
+ * step +-1, every q inside grid_shape).  q -> source taps along each source axis k, then clipped to [0, n_k - 1]:
+ *   taps != NULL (separable transform): source axis k reads taps[tap_off[k] + q[tap_grid[k]]] (device array of n_taps
+ *     entries built on the host from torch's own coordinates; its indices are not range-checked here);
+ *   taps == NULL (general): coordinate k = matrix[4k] q0 + matrix[4k+1] q1 + matrix[4k+2] q2 + matrix[4k+3] in fp64.
+ * NEAREST rounds half to even and copies one voxel; BILINEAR is trilinear in fp32 with the taps' weights. */
+#define MVTB_RESAMPLE_BILINEAR 0
+#define MVTB_RESAMPLE_NEAREST 1
+typedef struct mvtb_resample_tap {
+    int32_t i0, i1;          /* source indices of the low and high tap (i1 = min(i0 + 1, n - 1); nearest reads i0) */
+    float w0, w1;            /* their weights */
+} mvtb_resample_tap;
+typedef struct mvtb_resample_geom {
+    int32_t in_shape[3];     /* source (H, W, D) */
+    int32_t grid_shape[3];   /* Spacingd's output grid */
+    int32_t out_shape[3];    /* (s0, s1, s2) */
+    int32_t axis[3], base[3], step[3];
+    int32_t mode;            /* MVTB_RESAMPLE_* */
+    int32_t n_taps;
+    int32_t tap_grid[3], tap_off[3];
+    const mvtb_resample_tap* taps;
+    double matrix[12];
+} mvtb_resample_geom;
+int mvtb_resample_f32(const float* in, float* out, int n_volumes, const mvtb_resample_geom* geom, void* stream);
+
 /* WrapArtifact (F:503-515) on (C,H,W,D) when H, W and D are all even: the image-domain fold
  * out = prod_axes (c0 + s c1 Roll_{N/2}) x, c0=(1+alpha)/2, c1=(1-alpha)/2, s=(-1)^(N/2)
  * (SURVEY A.3).  Returns MVTB_EUNSUPPORTED for an odd axis (use the chain). in != out. */

@@ -39,6 +39,30 @@ class SpParams(C.Structure):
     _fields_ = [("p", C.c_float), ("seed", C.c_uint64), ("offset", C.c_uint64)]
 
 
+RESAMPLE_BILINEAR, RESAMPLE_NEAREST = 0, 1
+
+
+class ResampleTap(C.Structure):
+    _fields_ = [("i0", C.c_int32), ("i1", C.c_int32), ("w0", C.c_float), ("w1", C.c_float)]
+
+
+class ResampleGeom(C.Structure):
+    _fields_ = [
+        ("in_shape", C.c_int32 * 3),
+        ("grid_shape", C.c_int32 * 3),
+        ("out_shape", C.c_int32 * 3),
+        ("axis", C.c_int32 * 3),
+        ("base", C.c_int32 * 3),
+        ("step", C.c_int32 * 3),
+        ("mode", C.c_int32),
+        ("n_taps", C.c_int32),
+        ("tap_grid", C.c_int32 * 3),
+        ("tap_off", C.c_int32 * 3),
+        ("taps", C.c_void_p),
+        ("matrix", C.c_double * 12),
+    ]
+
+
 class MvtbError(RuntimeError):
     def __init__(self, code, text):
         super().__init__(f"libmvtb error {code}: {text}")
@@ -77,6 +101,7 @@ _SYMBOLS = {
                                      C.POINTER(C.c_int32), C.c_int, C.c_void_p]),
     "mvtb_crop_flip_batch_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                            C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mvtb_resample_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(ResampleGeom), C.c_void_p]),
     "mvtb_wrap_fold_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p]),
     "mvtb_wrap_odd_last_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p]),
     "mvtb_plan_profile": (C.c_int, [C.c_void_p, C.c_int]),

@@ -6,7 +6,9 @@
 // oracle/monai_spatial.py restates them).  Crop then flip is one gather:
 //     out[c][i][j][k] = in[c][o0 + (f0 ? s0-1-i : i)][o1 + (f1 ? s1-1-j : j)][o2 + (f2 ? s2-1-k : k)]
 // 8 B/voxel of the crop, nothing else; the host draws the offsets and the flip in MONAI's order (mvtb/spatial.py).
+// The resampling in front of them (Spacingd -> Orientationd) is k_resample (resample.cuh).
 #include "mvtb_common.cuh"
+#include "resample.cuh"
 
 namespace mvtb {
 
@@ -117,6 +119,66 @@ extern "C" int mvtb_crop_flip_batch_f32(const float* in, float* out, int n_sampl
     if (blocks > 148 * 16) blocks = 148 * 16;
     MVTB_LAUNCH(k_crop_flip_batch, dim3((unsigned)blocks), dim3(256), 0, stream, in, out, g, rows_per_sample, g.in_chan * n_channels,
                 offsets_dev, flips_dev, rows);
+    MVTB_CUDA(cudaGetLastError());
+    return MVTB_OK;
+}
+
+static bool is_perm3(const int32_t* p) {
+    return p[0] >= 0 && p[0] < 3 && p[1] >= 0 && p[1] < 3 && p[2] >= 0 && p[2] < 3 && p[0] != p[1] && p[0] != p[2] && p[1] != p[2];
+}
+
+extern "C" int mvtb_resample_f32(const float* in, float* out, int n_volumes, const mvtb_resample_geom* geom, void* stream) {
+    if (!in || !out || !geom) { set_error("resample: null argument"); return MVTB_EINVAL; }
+    if (in == out) { set_error("resample: in-place is not supported"); return MVTB_EINVAL; }
+    const mvtb_resample_geom& G = *geom;
+    if (n_volumes < 0) { set_error("resample: negative volume count"); return MVTB_EINVAL; }
+    if (G.mode != MVTB_RESAMPLE_BILINEAR && G.mode != MVTB_RESAMPLE_NEAREST) { set_error("resample: unknown mode %d", G.mode); return MVTB_EINVAL; }
+    for (int a = 0; a < 3; ++a)
+        if (G.in_shape[a] < 1 || G.grid_shape[a] < 1 || G.out_shape[a] < 0) {
+            set_error("resample: axis %d: source %d, grid %d, output %d", a, G.in_shape[a], G.grid_shape[a], G.out_shape[a]);
+            return MVTB_EINVAL;
+        }
+    if ((long long)G.in_shape[0] * G.in_shape[1] * G.in_shape[2] > 0x7fffffffLL) { set_error("resample: source volume over 2^31 voxels"); return MVTB_EINVAL; }
+    if (!is_perm3(G.axis)) { set_error("resample: axis is not a permutation of (0, 1, 2)"); return MVTB_EINVAL; }
+    for (int g = 0; g < 3; ++g) {
+        const long long n = G.out_shape[G.axis[g]], last = (long long)G.base[g] + (long long)G.step[g] * (n - 1);
+        if ((G.step[g] != 1 && G.step[g] != -1) || (n > 0 && (G.base[g] < 0 || G.base[g] >= G.grid_shape[g] || last < 0 || last >= G.grid_shape[g]))) {
+            set_error("resample: grid axis %d: base %d step %d over %lld outputs leaves [0, %d)", g, G.base[g], G.step[g], n, G.grid_shape[g]);
+            return MVTB_EINVAL;
+        }
+    }
+    ResampleDev d;
+    d.in_vol = (long long)G.in_shape[0] * G.in_shape[1] * G.in_shape[2];
+    for (int a = 0; a < 3; ++a) d.in_n[a] = G.in_shape[a];
+    d.in_stride[0] = G.in_shape[1] * G.in_shape[2]; d.in_stride[1] = G.in_shape[2]; d.in_stride[2] = 1;
+    d.s0 = G.out_shape[0]; d.s1 = G.out_shape[1]; d.s2 = G.out_shape[2];
+    d.taps = G.taps;
+    if (G.taps) {
+        if (!is_perm3(G.tap_grid)) { set_error("resample: tap_grid is not a permutation of (0, 1, 2)"); return MVTB_EINVAL; }
+        for (int k = 0; k < 3; ++k) {
+            const int g = G.tap_grid[k];
+            if (G.tap_off[k] < 0 || (long long)G.tap_off[k] + G.grid_shape[g] > G.n_taps) {
+                set_error("resample: source axis %d: taps [%d, %d) outside the %d entries", k, G.tap_off[k], G.tap_off[k] + G.grid_shape[g], G.n_taps);
+                return MVTB_EINVAL;
+            }
+            d.ax[k] = G.axis[g]; d.base[k] = G.tap_off[k] + G.base[g]; d.step[k] = G.step[g];
+        }
+    } else {
+        for (int i = 0; i < 12; ++i)
+            if (!std::isfinite(G.matrix[i])) { set_error("resample: matrix entry %d is not finite", i); return MVTB_EINVAL; }
+        for (int g = 0; g < 3; ++g) { d.ax[g] = G.axis[g]; d.base[g] = G.base[g]; d.step[g] = G.step[g]; }
+        for (int k = 0; k < 3; ++k)
+            for (int i = 0; i < 4; ++i) d.m[k][i] = G.matrix[4 * k + i];
+    }
+    const long long rows = (long long)n_volumes * d.s0 * d.s1;
+    if (rows == 0 || d.s2 == 0) return MVTB_OK;
+    long long blocks = (rows + 7) / 8;                      // one warp per output row, 8 warps per CTA
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    const bool nearest = G.mode == MVTB_RESAMPLE_NEAREST;
+    if (G.taps && nearest) { auto kern = k_resample<true, true>; MVTB_LAUNCH(kern, dim3((unsigned)blocks), dim3(256), 0, stream, in, out, d, rows); }
+    else if (G.taps) { auto kern = k_resample<true, false>; MVTB_LAUNCH(kern, dim3((unsigned)blocks), dim3(256), 0, stream, in, out, d, rows); }
+    else if (nearest) { auto kern = k_resample<false, true>; MVTB_LAUNCH(kern, dim3((unsigned)blocks), dim3(256), 0, stream, in, out, d, rows); }
+    else { auto kern = k_resample<false, false>; MVTB_LAUNCH(kern, dim3((unsigned)blocks), dim3(256), 0, stream, in, out, d, rows); }
     MVTB_CUDA(cudaGetLastError());
     return MVTB_OK;
 }
