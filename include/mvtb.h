@@ -229,6 +229,23 @@ typedef struct mvtb_resample_geom {
 } mvtb_resample_geom;
 int mvtb_resample_f32(const float* in, float* out, int n_volumes, const mvtb_resample_geom* geom, void* stream);
 
+/* The decode half of LoadImaged -> AsChannelFirstd: a NIfTI-1/2 payload already on the device (raw: the vox_offset-th byte
+ * of the file, aligned to its element size) -> out (C, X, Y, Z) C-contiguous float32, out[c][i][j][k] = file element
+ * ((c Z + k) Y + j) X + i.  dims = (X, Y, Z, C), a host array; X Y Z <= 2^31.  datatype: a NIfTI code below (others:
+ * MVTB_EUNSUPPORTED); swap_bytes: the file's byte order is not the device's.  scaled = 0: float(raw), rounded to nearest
+ * even; scaled != 0: raw * slope + inter in float32 (8/16-bit integers, float32) or float64 (32-bit integers, float64),
+ * the multiply and the add rounded separately, then rounded to float32.  raw != out. */
+#define MVTB_NIFTI_UINT8 2
+#define MVTB_NIFTI_INT16 4
+#define MVTB_NIFTI_INT32 8
+#define MVTB_NIFTI_FLOAT32 16
+#define MVTB_NIFTI_FLOAT64 64
+#define MVTB_NIFTI_INT8 256
+#define MVTB_NIFTI_UINT16 512
+#define MVTB_NIFTI_UINT32 768
+int mvtb_nifti_decode_f32(const void* raw, float* out, int32_t datatype, int32_t swap_bytes, const int64_t* dims, double slope,
+                          double inter, int32_t scaled, void* stream);
+
 /* WrapArtifact (F:503-515) on (C,H,W,D) when H, W and D are all even: the image-domain fold
  * out = prod_axes (c0 + s c1 Roll_{N/2}) x, c0=(1+alpha)/2, c1=(1-alpha)/2, s=(-1)^(N/2)
  * (SURVEY A.3).  Returns MVTB_EUNSUPPORTED for an odd axis (use the chain). in != out. */

@@ -56,12 +56,17 @@ class SelectChanneld(MapTransform):
 
 
 class ConvertToMultiChannelBasedOnBratsClassesd(MapTransform):
-    """BraTS labels -> (TC, WT, ET) float32 channels (F:61-87)."""
+    """BraTS labels -> (TC, WT, ET) float32 channels (F:61-87).  A CUDA tensor (mvtb.nifti.LoadImaged's output) stays on
+    its device and comes back as CUDA float32."""
 
     def __call__(self, data):
         d = dict(data)
         for key in self.keys:
             lab = d[key]
+            if isinstance(lab, torch.Tensor) and lab.is_cuda:
+                tc = (lab == 2) | (lab == 3)
+                d[key] = torch.stack([tc, tc | (lab == 1), lab == 2], dim=0).to(torch.float32)
+                continue
             tc = np.logical_or(lab == 2, lab == 3)
             wt = np.logical_or(tc, lab == 1)
             et = lab == 2

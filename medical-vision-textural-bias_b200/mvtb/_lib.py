@@ -102,6 +102,8 @@ _SYMBOLS = {
     "mvtb_crop_flip_batch_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                            C.c_void_p, C.c_void_p, C.c_void_p]),
     "mvtb_resample_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(ResampleGeom), C.c_void_p]),
+    "mvtb_nifti_decode_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.c_double, C.c_double,
+                                        C.c_int32, C.c_void_p]),
     "mvtb_wrap_fold_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p]),
     "mvtb_wrap_odd_last_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p]),
     "mvtb_plan_profile": (C.c_int, [C.c_void_p, C.c_int]),

@@ -14,6 +14,10 @@
 #define MVTB_DYN_SMEM(name) unsigned char* name = cuemu::g_dyn_smem
 #define MVTB_UNROLL
 #define MVTB_UNROLL_N(n)
+// double-precision intrinsics the emulator lacks (nifti.cuh); volatile keeps g++ from contracting them into an FMA
+static inline float __double2float_rn(double d) { return (float)d; }
+static inline double __dmul_rn(double a, double b) { volatile double r = a * b; return r; }
+static inline double __dadd_rn(double a, double b) { volatile double r = a + b; return r; }
 #else
 #include <cuda_runtime.h>
 #define MVTB_LAUNCH(kern, grid, block, smem, stream, ...) \

@@ -6,8 +6,10 @@
 // oracle/monai_spatial.py restates them).  Crop then flip is one gather:
 //     out[c][i][j][k] = in[c][o0 + (f0 ? s0-1-i : i)][o1 + (f1 ? s1-1-j : j)][o2 + (f2 ? s2-1-k : k)]
 // 8 B/voxel of the crop, nothing else; the host draws the offsets and the flip in MONAI's order (mvtb/spatial.py).
-// The resampling in front of them (Spacingd -> Orientationd) is k_resample (resample.cuh).
+// The resampling in front of them (Spacingd -> Orientationd) is k_resample (resample.cuh); in front of that, the NIfTI
+// payload is decoded to channel-first float32 by k_nifti_decode (nifti.cuh).
 #include "mvtb_common.cuh"
+#include "nifti.cuh"
 #include "resample.cuh"
 
 namespace mvtb {
@@ -179,6 +181,58 @@ extern "C" int mvtb_resample_f32(const float* in, float* out, int n_volumes, con
     else if (G.taps) { auto kern = k_resample<true, false>; MVTB_LAUNCH(kern, dim3((unsigned)blocks), dim3(256), 0, stream, in, out, d, rows); }
     else if (nearest) { auto kern = k_resample<false, true>; MVTB_LAUNCH(kern, dim3((unsigned)blocks), dim3(256), 0, stream, in, out, d, rows); }
     else { auto kern = k_resample<false, false>; MVTB_LAUNCH(kern, dim3((unsigned)blocks), dim3(256), 0, stream, in, out, d, rows); }
+    MVTB_CUDA(cudaGetLastError());
+    return MVTB_OK;
+}
+
+// NIfTI datatype code -> element bytes (0: not supported)
+static int nifti_bytes(int32_t datatype) {
+    switch (datatype) {
+        case MVTB_NIFTI_UINT8: case MVTB_NIFTI_INT8: return 1;
+        case MVTB_NIFTI_INT16: case MVTB_NIFTI_UINT16: return 2;
+        case MVTB_NIFTI_INT32: case MVTB_NIFTI_UINT32: case MVTB_NIFTI_FLOAT32: return 4;
+        case MVTB_NIFTI_FLOAT64: return 8;
+        default: return 0;
+    }
+}
+
+template <typename T>
+static void nifti_launch(const void* raw, float* out, const NiftiDev& d, void* stream) {
+    const long long planes = d.C * d.Y;
+    const dim3 grid((unsigned)((d.X + MVTB_NIFTI_TILE - 1) / MVTB_NIFTI_TILE), (unsigned)((d.Z + MVTB_NIFTI_TILE - 1) / MVTB_NIFTI_TILE),
+                    (unsigned)(planes < 65535 ? planes : 65535));
+    auto kern = k_nifti_decode<T>;
+    MVTB_LAUNCH(kern, grid, dim3(MVTB_NIFTI_TILE, MVTB_NIFTI_ROWS), 0, stream, (const T*)raw, out, d);
+}
+
+extern "C" int mvtb_nifti_decode_f32(const void* raw, float* out, int32_t datatype, int32_t swap_bytes, const int64_t* dims, double slope,
+                                     double inter, int32_t scaled, void* stream) {
+    if (!raw || !out || !dims) { set_error("nifti_decode: null argument"); return MVTB_EINVAL; }
+    if (raw == (const void*)out) { set_error("nifti_decode: in-place is not supported"); return MVTB_EINVAL; }
+    const int bytes = nifti_bytes(datatype);
+    if (!bytes) { set_error("nifti_decode: NIfTI datatype %d is not supported", datatype); return MVTB_EUNSUPPORTED; }
+    if ((uintptr_t)raw % bytes) { set_error("nifti_decode: payload address not aligned to its %d-byte elements", bytes); return MVTB_EINVAL; }
+    for (int a = 0; a < 4; ++a)
+        if (dims[a] < 1) { set_error("nifti_decode: dims[%d] = %lld", a, (long long)dims[a]); return MVTB_EINVAL; }
+    if (dims[0] > 0x7fffffffLL || dims[1] > 0x7fffffffLL || dims[2] > 0x7fffffffLL || dims[0] * dims[1] * dims[2] > 0x7fffffffLL) {
+        set_error("nifti_decode: %lld x %lld x %lld voxels per channel, over 2^31", (long long)dims[0], (long long)dims[1], (long long)dims[2]);
+        return MVTB_EINVAL;
+    }
+    NiftiDev d;
+    d.X = (int)dims[0]; d.Y = (int)dims[1]; d.Z = (int)dims[2]; d.C = dims[3];
+    d.swap = swap_bytes != 0 && bytes > 1;
+    d.scaled = scaled != 0;
+    d.s32 = (float)slope; d.i32 = (float)inter; d.s64 = slope; d.i64 = inter;
+    switch (datatype) {
+        case MVTB_NIFTI_UINT8: nifti_launch<uint8_t>(raw, out, d, stream); break;
+        case MVTB_NIFTI_INT8: nifti_launch<int8_t>(raw, out, d, stream); break;
+        case MVTB_NIFTI_INT16: nifti_launch<int16_t>(raw, out, d, stream); break;
+        case MVTB_NIFTI_UINT16: nifti_launch<uint16_t>(raw, out, d, stream); break;
+        case MVTB_NIFTI_INT32: nifti_launch<int32_t>(raw, out, d, stream); break;
+        case MVTB_NIFTI_UINT32: nifti_launch<uint32_t>(raw, out, d, stream); break;
+        case MVTB_NIFTI_FLOAT32: nifti_launch<float>(raw, out, d, stream); break;
+        default: nifti_launch<double>(raw, out, d, stream); break;
+    }
     MVTB_CUDA(cudaGetLastError());
     return MVTB_OK;
 }
