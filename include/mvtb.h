@@ -121,6 +121,16 @@ typedef struct mvtb_sp_params {
 int mvtb_kspace_chain_ex_f32(mvtb_plan* plan, const float* in, float* out, int n_volumes,
                              const mvtb_chain_desc* desc, int n_desc, const float* pre_abt,
                              float* minmax_out, int vols_per_sample, const mvtb_sp_params* sp, void* stream);
+/* mvtb_kspace_chain_ex_f32 with the distance between samples' Philox span counters set: span s of sample i uses counter
+ * offset + i * sample_stride + s (0 = ceil(voxels per sample / MVTB_SP_SPAN), which is mvtb_kspace_chain_ex_f32; a nonzero
+ * stride must not be below that span count).  One call over a batch then draws the hits that one call per sample would draw
+ * with `offset` advanced by sample_stride between calls -- SaltAndPepper(rng="philox-sparse") advances it by
+ * ceil(voxels / 256) per call.  The select pass runs where mvtb_kspace_chain_ex_f32 runs it (fused into the inverse kernel
+ * when it can be). */
+int mvtb_kspace_chain_ex_strided_f32(mvtb_plan* plan, const float* in, float* out, int n_volumes,
+                                     const mvtb_chain_desc* desc, int n_desc, const float* pre_abt,
+                                     float* minmax_out, int vols_per_sample, const mvtb_sp_params* sp,
+                                     uint64_t sample_stride, void* stream);
 
 /* sum over the full (unshifted, unnormalised) spectrum of log(|k| + 1e-10) per volume, into
  * device double[n_volumes]; the caller divides by the volume size and multiplies by 2.5
@@ -200,6 +210,21 @@ int mvtb_crop_flip_f32(const float* in, float* out, int n_channels, const int32_
  * flips_dev[n_samples] are int32 arrays ON THE DEVICE (windows are not range-checked). */
 int mvtb_crop_flip_batch_f32(const float* in, float* out, int n_samples, int n_channels, const int32_t* in_shape,
                              const int32_t* out_shape, const int32_t* offsets_dev, const int32_t* flips_dev, void* stream);
+/* The same gather for a batch whose samples come from a ragged cache (the training loader's device-resident sample cache):
+ *   out[b][c] = flip_b(entry[entry_dev[b]][channels[c]][start_b : start_b + out_shape])
+ * Entry e holds n_channels_in channels of spatial shape entry_shape_dev[3e .. 3e+2], C-contiguous, starting at element
+ * entry_offset_dev[e] of `cache`.  channels: host array of n_channels_out (<= MVTB_GATHER_MAX_CHANNELS) indices into the
+ * stored channels, in any order, or NULL for all of them (then n_channels_out == n_channels_in): a SelectChanneld in front
+ * of the crop costs nothing, the unselected channels are never read.  out_shape: host, every axis >= 1.  out: (n_samples,
+ * n_channels_out, s0, s1, s2), cache != out.  entry_dev[n_samples], starts_dev[3 n_samples] and flips_dev[n_samples] (bit a =
+ * spatial axis a; bits above 2 are ignored) are int32 arrays ON THE DEVICE, as are the int64 entry_offset_dev and the int32
+ * entry_shape_dev tables: none of them is checked here.  The caller guarantees that every entry index is valid and that
+ * 0 <= start_b and start_b + out_shape <= the entry's shape on every axis (mvtb/train_stage.py checks each window on the
+ * host before it uploads them). */
+#define MVTB_GATHER_MAX_CHANNELS 8
+int mvtb_crop_flip_gather_f32(const float* cache, float* out, int n_samples, int n_channels_out, const int64_t* entry_offset_dev,
+                              const int32_t* entry_shape_dev, int n_channels_in, const int32_t* channels, const int32_t* out_shape,
+                              const int32_t* entry_dev, const int32_t* starts_dev, const int32_t* flips_dev, void* stream);
 
 /* Spacingd -> Orientationd (MONAI 0.5, 127_...FLAIR.py:120-129: pixdim (1.5, 1.5, 2.0), modes bilinear / nearest,
  * border padding, align_corners=False; then axcodes "RAS"), optionally followed by a crop and flip, as one gather from

@@ -81,6 +81,8 @@ _SYMBOLS = {
                                            C.c_void_p, C.c_int, C.c_float, C.c_uint64, C.c_uint64, C.c_void_p]),
     "mvtb_kspace_chain_ex_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(ChainDesc), C.c_int, C.c_void_p,
                                            C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "mvtb_kspace_chain_ex_strided_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(ChainDesc), C.c_int,
+                                                   C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p]),
     "mvtb_kspace_logabs_sum_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "mvtb_minmax_f32": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p]),
     "mvtb_salt_pepper_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_uint64, C.c_uint64,
@@ -101,6 +103,9 @@ _SYMBOLS = {
                                      C.POINTER(C.c_int32), C.c_int, C.c_void_p]),
     "mvtb_crop_flip_batch_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                            C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mvtb_crop_flip_gather_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
+                                            C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p]),
     "mvtb_resample_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(ResampleGeom), C.c_void_p]),
     "mvtb_nifti_decode_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.c_double, C.c_double,
                                         C.c_int32, C.c_void_p]),

@@ -887,6 +887,7 @@ static int bl_run(mvtb_plan* p, const float* in, float* out, int n_volumes, cons
         if (bps > 0x7fffffffull || B >= (1ull << 28) || (unsigned long long)ia.A >= (1ull << 28)) fuse = false;
         else {
             ia.bps = (unsigned)bps;
+            ia.stride = sp->stride ? sp->stride : bps;
             const int lag = p->is_lag >= 0 ? p->is_lag : 2 * p->num_sms + 8;
             const int spread = (int)((long long)ia.A * p->is_spread_pct / 100);
             is_build_pattern(ia.A, (int)B, lag, spread, pattern, &max_back);
@@ -989,6 +990,7 @@ static int bl_run(mvtb_plan* p, const float* in, float* out, int n_volumes, cons
             sa.vol_n = (unsigned long long)p->vol_real;
             sa.n_per_sample = (unsigned long long)vps * p->vol_real;
             sa.bps = (unsigned)tc_bps;
+            sa.stride = sp->stride ? sp->stride : tc_bps;
             sa.s_base = v0 / vps;
             sa.table = (const unsigned*)((const unsigned char*)dvp + tab_off);
             const double l2q = log2(1.0 - (double)sp->p);
@@ -1200,6 +1202,7 @@ static int bl_run(mvtb_plan* p, const float* in, float* out, int n_volumes, cons
                 ta.offset = sp->offset;
                 ta.n_per_sample = (unsigned long long)vps * p->vol_real;
                 ta.bps = (unsigned)tc_bps;
+                ta.stride = sp->stride ? sp->stride : tc_bps;
                 ta.s_base = v0 / vps;
                 if (dprof_i && getenv("MVTB_TC_PROF")) ta.prof = dprof_i + 2048;
                 auto kern = k_bl_inv_tc<NF, 3>;

@@ -37,6 +37,7 @@ struct IsArgs {
     unsigned long long seed, offset;
     unsigned long long n_per_sample;
     unsigned bps;                // spans of MVTB_SP_SPAN voxels per sample
+    unsigned long long stride;   // Philox span counters from one sample to the next (>= bps)
     float* minmax;               // 2 floats per sample of the call
     int debug;                   // measurements: 1 = select tiles do no work, 2 = ... and do not wait, 4 = inverse tiles skip the fences, 8 = hits stored as found
 };
@@ -139,7 +140,7 @@ k_bl_inv_sp(const cf* __restrict__ Y, float* __restrict__ out, BlGeom g, const B
             const unsigned span = ((unsigned)j * 8u + (unsigned)(tid >> 5)) * kIsSpansPerWarp;
             if (span < a.bps)
                 sp_walk_spans<kIsSpansPerWarp>(out + (size_t)s * a.n_per_sample, a.n_per_sample, span, a.bps,
-                                               a.offset + (unsigned long long)(a.s_base + s) * a.bps + span, key, sT, a.inv_log2q,
+                                               a.offset + (unsigned long long)(a.s_base + s) * a.stride + span, key, sT, a.inv_log2q,
                                                lo, hi, tid & 31, (a.debug & 8) ? nullptr : s_stage[tid >> 5]);
         }
     }

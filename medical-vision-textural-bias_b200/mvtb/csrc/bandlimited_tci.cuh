@@ -68,6 +68,7 @@ struct TciArgs {
     float inv_log2q;
     unsigned long long seed, offset, n_per_sample;
     unsigned bps;                // spans per sample
+    unsigned long long stride;   // Philox span counters from one sample to the next (>= bps)
     int s_base;                  // index of the launch's first sample in the call
     int debug;                   // MVTB_TCI_DEBUG, measurements: 1 = the select warps wait but do not walk, 2 = no fence before the counters (unsafe)
     int* status;
@@ -227,7 +228,7 @@ k_bl_inv_tc(TciArgs a) {
             // bound by its dependent chains (Philox, table search, prefix sum) and interleaved chains overlap them
             for (unsigned span = gsw * kTciSelSpans; span < a.bps; span += nsw * kTciSelSpans)
                 sp_walk_spans<kTciSelSpans>(a.out + (size_t)sidx * a.n_per_sample, a.n_per_sample, span, a.bps,
-                                            a.offset + (unsigned long long)(a.s_base + sidx) * a.bps + span, key, s_spT, a.inv_log2q, slo, shi, lane);
+                                            a.offset + (unsigned long long)(a.s_base + sidx) * a.stride + span, key, s_spT, a.inv_log2q, slo, shi, lane);
         }
     } else if (warp < kTciWarpEpi0) {
         // ------------------------------------------------------------ A builders: group = tile parity, thread = column of the tile
@@ -470,6 +471,7 @@ struct SpBitsArgs {
     unsigned long long vol_n;    // voxels per volume
     unsigned long long n_per_sample;
     unsigned bps;                // spans per sample
+    unsigned long long stride;   // Philox span counters from one sample to the next (>= bps)
     int s_base;                  // index of the launch's first sample in the call
     const unsigned* table;
     float inv_log2q;
@@ -502,7 +504,7 @@ k_sp_bits(SpBitsArgs a) {
         long long row0l = rel0 / NC;
         if (rel0 - row0l * NC < 0) --row0l;
         const int row0 = (int)row0l, col0 = (int)(rel0 - row0l * NC);
-        sp_walk_span_cb(len, a.offset + (unsigned long long)(a.s_base + s) * a.bps + span, key, sT, a.inv_log2q, lane,
+        sp_walk_span_cb(len, a.offset + (unsigned long long)(a.s_base + s) * a.stride + span, key, sT, a.inv_log2q, lane,
                         [&](int pos, unsigned coin) {
                             int c = col0 + pos, j = row0;
                             while (c >= NC) { c -= NC; ++j; }

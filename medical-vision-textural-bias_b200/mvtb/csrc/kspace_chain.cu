@@ -833,9 +833,9 @@ extern "C" int mvtb_kspace_chain_f32(mvtb_plan* p, const float* in, float* out, 
     return chain_impl(p, in, out, n_volumes, desc, n_desc, minmax_out, vols_per_sample, stream, nullptr, nullptr);
 }
 
-extern "C" int mvtb_kspace_chain_ex_f32(mvtb_plan* p, const float* in, float* out, int n_volumes,
-                                        const mvtb_chain_desc* desc, int n_desc, const float* pre_abt, float* minmax_out,
-                                        int vols_per_sample, const mvtb_sp_params* spp, void* stream) {
+extern "C" int mvtb_kspace_chain_ex_strided_f32(mvtb_plan* p, const float* in, float* out, int n_volumes,
+                                                const mvtb_chain_desc* desc, int n_desc, const float* pre_abt, float* minmax_out,
+                                                int vols_per_sample, const mvtb_sp_params* spp, uint64_t sample_stride, void* stream) {
     if (!spp) return chain_impl(p, in, out, n_volumes, desc, n_desc, minmax_out, vols_per_sample, stream, nullptr, pre_abt);
     const float prob = spp->p;
     if (!p || !minmax_out) { set_error("chain_sp: null plan or minmax_out"); return MVTB_EINVAL; }
@@ -845,8 +845,12 @@ extern "C" int mvtb_kspace_chain_ex_f32(mvtb_plan* p, const float* in, float* ou
         return MVTB_EINVAL;
     }
     if (n_volumes / vols_per_sample > 65535) { set_error("chain_sp: more than 65535 samples in one call"); return MVTB_EUNSUPPORTED; }
+    if (sample_stride && sample_stride < ((unsigned long long)vols_per_sample * p->vol_real + MVTB_SP_SPAN - 1) / MVTB_SP_SPAN) {
+        set_error("chain_sp: sample_stride %llu is below a sample's span count", (unsigned long long)sample_stride);
+        return MVTB_EINVAL;
+    }
     SpFuse sp;
-    sp.p = prob; sp.seed = spp->seed; sp.offset = spp->offset; sp.done = false;
+    sp.p = prob; sp.seed = spp->seed; sp.offset = spp->offset; sp.stride = sample_stride; sp.done = false;
     int rc = chain_impl(p, in, out, n_volumes, desc, n_desc, minmax_out, vols_per_sample, stream, &sp, pre_abt);
     if (rc != MVTB_OK || sp.done || prob == 0.f || n_volumes == 0) return rc;
     // any other path: the select pass follows as its own kernel (same Philox counters, same result)
@@ -857,7 +861,13 @@ extern "C" int mvtb_kspace_chain_ex_f32(mvtb_plan* p, const float* in, float* ou
     rc = plan_stage_upload(p, host_table, sizeof(host_table), stream, &dtab);
     if (rc != MVTB_OK) return rc;
     return sparse_sp_launch(out, (size_t)vols_per_sample * p->vol_real, n_volumes / vols_per_sample, spp->seed, spp->offset, prob,
-                            minmax_out, (const unsigned*)dtab, stream);
+                            minmax_out, (const unsigned*)dtab, stream, sample_stride);
+}
+
+extern "C" int mvtb_kspace_chain_ex_f32(mvtb_plan* p, const float* in, float* out, int n_volumes,
+                                        const mvtb_chain_desc* desc, int n_desc, const float* pre_abt, float* minmax_out,
+                                        int vols_per_sample, const mvtb_sp_params* spp, void* stream) {
+    return mvtb_kspace_chain_ex_strided_f32(p, in, out, n_volumes, desc, n_desc, pre_abt, minmax_out, vols_per_sample, spp, 0, stream);
 }
 
 extern "C" int mvtb_kspace_chain_sp_f32(mvtb_plan* p, const float* in, float* out, int n_volumes,

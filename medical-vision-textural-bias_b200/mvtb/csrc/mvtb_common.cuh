@@ -95,12 +95,14 @@ __device__ __forceinline__ void cp_async_wait() {
 // ---------------------------------------------------------------- per-axis FFT description
 struct DescDev;
 // voxel_ops.cu: the geometric-gap sampler on its own (table_dev already holds mvtb_sparse_table(p))
+// sample_stride: Philox span counters between consecutive samples, 0 = the sample's own span count
 int sparse_sp_launch(float* x, size_t n_per_sample, int n_samples, uint64_t seed, uint64_t offset, float p,
-                     const float* minmax, const unsigned* table_dev, void* stream);
+                     const float* minmax, const unsigned* table_dev, void* stream, uint64_t sample_stride = 0);
 // salt-and-pepper to run behind the chain (mvtb_kspace_chain_sp_f32); `done` is set by the path that fused it
 struct SpFuse {
     float p;
     unsigned long long seed, offset;
+    unsigned long long stride;   // Philox span counters from one sample to the next; 0 = the sample's span count
     bool done;
 };
 #define MVTB_MAX_STAGES 12

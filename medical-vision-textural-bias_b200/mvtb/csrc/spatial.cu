@@ -70,9 +70,87 @@ k_crop_flip_batch(const float* __restrict__ in, float* __restrict__ out, CropGeo
     }
 }
 
+// the same gather from a ragged cache (the training loader's DeviceCache): sample b reads cache entry entry[b], whose
+// spatial shape and first element come from the entry tables, so every sample finds its own row and plane pitch; the
+// output channels are the entry's channels g.ch[0 .. n_out_ch) (a SelectChanneld folded into the gather)
+struct GatherGeom {
+    int s0, s1, s2;        // output shape
+    int ch[MVTB_GATHER_MAX_CHANNELS];
+};
+
+__global__ void __launch_bounds__(256)
+k_crop_flip_gather(const float* __restrict__ cache, float* __restrict__ out, GatherGeom g, long long rows_per_sample,
+                   const long long* __restrict__ entry_offset, const int* __restrict__ entry_shape, const int* __restrict__ entry,
+                   const int* __restrict__ starts, const int* __restrict__ flips, long long n_rows_total) {
+    const int lane = threadIdx.x & 31;
+    const long long wid = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long rr = wid; rr < n_rows_total; rr += nw) {
+        const long long b = rr / rows_per_sample, r = rr - b * rows_per_sample;
+        const int e = __ldg(entry + b);
+        const int iw = __ldg(entry_shape + 3 * e + 1), id = __ldg(entry_shape + 3 * e + 2);
+        const long long in_chan = (long long)__ldg(entry_shape + 3 * e) * iw * id;
+        const int o0 = __ldg(starts + 3 * b), o1 = __ldg(starts + 3 * b + 1), o2 = __ldg(starts + 3 * b + 2), fl = __ldg(flips + b);
+        const int c = (int)(r / ((long long)g.s0 * g.s1));
+        const int rem = (int)(r - (long long)c * g.s0 * g.s1);
+        const int i = rem / g.s1, j = rem - i * g.s1;
+        const int si = o0 + ((fl & 1) ? g.s0 - 1 - i : i);
+        const int sj = o1 + ((fl & 2) ? g.s1 - 1 - j : j);
+        const float* src = cache + __ldg(entry_offset + e) + g.ch[c] * in_chan + ((long long)si * iw + sj) * id + o2;
+        float* dst = out + rr * g.s2;
+        if (fl & 4) {
+            for (int k = lane; k < g.s2; k += 32) dst[k] = src[g.s2 - 1 - k];
+        } else {
+            for (int k = lane; k < g.s2; k += 32) dst[k] = src[k];
+        }
+    }
+}
+
 }  // namespace mvtb
 
 using namespace mvtb;
+
+extern "C" int mvtb_crop_flip_gather_f32(const float* cache, float* out, int n_samples, int n_channels_out, const int64_t* entry_offset_dev,
+                                         const int32_t* entry_shape_dev, int n_channels_in, const int32_t* channels,
+                                         const int32_t* out_shape, const int32_t* entry_dev, const int32_t* starts_dev,
+                                         const int32_t* flips_dev, void* stream) {
+    if (!cache || !out || !entry_offset_dev || !entry_shape_dev || !out_shape || !entry_dev || !starts_dev || !flips_dev) {
+        set_error("crop_flip_gather: null argument");
+        return MVTB_EINVAL;
+    }
+    if (cache == out) { set_error("crop_flip_gather: in-place is not supported"); return MVTB_EINVAL; }
+    if (n_samples < 0 || n_channels_out < 0 || n_channels_in < 0) { set_error("crop_flip_gather: negative count"); return MVTB_EINVAL; }
+    if (n_channels_out > MVTB_GATHER_MAX_CHANNELS) {
+        set_error("crop_flip_gather: %d output channels, at most %d", n_channels_out, MVTB_GATHER_MAX_CHANNELS);
+        return MVTB_EINVAL;
+    }
+    if (!channels && n_channels_out != n_channels_in) {
+        set_error("crop_flip_gather: channels = NULL selects all %d channels, not %d", n_channels_in, n_channels_out);
+        return MVTB_EINVAL;
+    }
+    GatherGeom g;
+    for (int c = 0; c < MVTB_GATHER_MAX_CHANNELS; ++c) g.ch[c] = 0;
+    for (int c = 0; c < n_channels_out; ++c) {
+        g.ch[c] = channels ? channels[c] : c;
+        if (g.ch[c] < 0 || g.ch[c] >= n_channels_in) {
+            set_error("crop_flip_gather: channel %d outside the %d stored channels", g.ch[c], n_channels_in);
+            return MVTB_EINVAL;
+        }
+    }
+    for (int a = 0; a < 3; ++a)
+        if (out_shape[a] < 1) { set_error("crop_flip_gather: output axis %d has size %d", a, out_shape[a]); return MVTB_EINVAL; }
+    g.s0 = out_shape[0]; g.s1 = out_shape[1]; g.s2 = out_shape[2];
+    const long long rows_per_sample = (long long)n_channels_out * g.s0 * g.s1;
+    const long long rows = rows_per_sample * n_samples;
+    if (rows == 0) return MVTB_OK;
+    long long blocks = (rows + 7) / 8;                      // 8 warps per CTA
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    MVTB_LAUNCH(k_crop_flip_gather, dim3((unsigned)blocks), dim3(256), 0, stream, cache, out, g, rows_per_sample,
+                (const long long*)entry_offset_dev, (const int*)entry_shape_dev, (const int*)entry_dev, (const int*)starts_dev,
+                (const int*)flips_dev, rows);
+    MVTB_CUDA(cudaGetLastError());
+    return MVTB_OK;
+}
 
 extern "C" int mvtb_crop_flip_f32(const float* in, float* out, int n_channels, const int32_t* in_shape, const int32_t* out_shape,
                                   const int32_t* offset, int flip_axes_mask, void* stream) {

@@ -224,7 +224,7 @@ static const int kSpThreadsSparse = 256;
 
 __global__ void __launch_bounds__(kSpThreadsSparse)
 k_salt_pepper_sparse(float* __restrict__ x, unsigned long long n_per_sample, unsigned spans_per_sample,
-                     const unsigned* __restrict__ table, float inv_log2q, uint64_t seed, uint64_t offset,
+                     const unsigned* __restrict__ table, float inv_log2q, uint64_t seed, uint64_t offset, uint64_t sample_stride,
                      const float* __restrict__ mm) {
     __shared__ unsigned sT[MVTB_SP_BLOCK];
     __shared__ unsigned short s_stage[kSpThreadsSparse / 32][kSpStageIters * 96];
@@ -238,7 +238,7 @@ k_salt_pepper_sparse(float* __restrict__ x, unsigned long long n_per_sample, uns
     key.x = (unsigned)seed;
     key.y = (unsigned)(seed >> 32);
     sp_walk_spans<1>(x + (size_t)smp * n_per_sample, n_per_sample, span, spans_per_sample,
-                     offset + (uint64_t)smp * spans_per_sample + span, key, sT, inv_log2q, lo, hi, threadIdx.x & 31,
+                     offset + (uint64_t)smp * sample_stride + span, key, sT, inv_log2q, lo, hi, threadIdx.x & 31,
                      s_stage[threadIdx.x >> 5]);
 }
 
@@ -380,16 +380,22 @@ extern "C" int mvtb_sparse_table(float p, unsigned* table_out) {
 
 namespace mvtb {
 int sparse_sp_launch(float* x, size_t n_per_sample, int n_samples, uint64_t seed, uint64_t offset, float p,
-                     const float* minmax, const unsigned* table_dev, void* stream) {
-    if (p == 0.f || n_samples == 0 || n_per_sample == 0) return MVTB_OK;   // T = 0 everywhere: no voxel is ever selected
+                     const float* minmax, const unsigned* table_dev, void* stream, uint64_t sample_stride) {
     const size_t sps = (n_per_sample + MVTB_SP_SPAN - 1) / MVTB_SP_SPAN;
+    if (sample_stride == 0) sample_stride = sps;
+    if (sample_stride < sps) {
+        set_error("salt_pepper_sparse: sample stride %llu below the %llu spans of a sample", (unsigned long long)sample_stride,
+                  (unsigned long long)sps);
+        return MVTB_EINVAL;
+    }
+    if (p == 0.f || n_samples == 0 || n_per_sample == 0) return MVTB_OK;   // T = 0 everywhere: no voxel is ever selected
     if (sps > 0x7fffffffull) { set_error("salt_pepper_sparse: sample too large"); return MVTB_EUNSUPPORTED; }
     const unsigned per_cta = (unsigned)(kSpThreadsSparse / 32);
     const unsigned gx = (unsigned)((sps + per_cta - 1) / per_cta);
     const double l2q = log2(1.0 - (double)p);          // -inf for p = 1: the guess is then 0 and the table decides
     const float inv_log2q = (l2q < 0.0 && l2q > -1e300) ? (float)(1.0 / l2q) : 0.f;
     MVTB_LAUNCH(k_salt_pepper_sparse, dim3(gx, (unsigned)n_samples), dim3(kSpThreadsSparse), 0, stream, x,
-                (unsigned long long)n_per_sample, (unsigned)sps, table_dev, inv_log2q, seed, offset, minmax);
+                (unsigned long long)n_per_sample, (unsigned)sps, table_dev, inv_log2q, seed, offset, sample_stride, minmax);
     MVTB_CUDA(cudaGetLastError());
     return MVTB_OK;
 }

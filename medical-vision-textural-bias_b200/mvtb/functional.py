@@ -209,7 +209,8 @@ def kspace_chain_ex(x: torch.Tensor, ndim_fft: int, descs: Sequence[_lib.ChainDe
                     sp: Optional[Tuple[float, int, int]] = None, want_minmax: bool = False, vols_per_sample: int = 1,
                     out: Optional[torch.Tensor] = None):
     """mvtb_kspace_chain_ex_f32: [intensity prologue map on the way in] -> chain -> [sparse salt-and-pepper on the way
-    out].  pre_abt: float32 CUDA tensor (n_volumes, 3) from intensity_coeffs(); sp: (p, seed, offset).
+    out].  pre_abt: float32 CUDA tensor (n_volumes, 3) from intensity_coeffs(); sp: (p, seed, offset[, sample_stride]), the
+    stride being the distance between samples' Philox span counters (mvtb_kspace_chain_ex_strided_f32; 0 = spans per sample).
     Returns y, or (y, minmax) when want_minmax or sp is given."""
     L = _lib.lib()
     if not x.is_cuda or x.dtype != torch.float32 or not x.is_contiguous():
@@ -229,9 +230,11 @@ def kspace_chain_ex(x: torch.Tensor, ndim_fft: int, descs: Sequence[_lib.ChainDe
     spp = None
     if sp is not None:
         spp = _lib.SpParams(float(sp[0]), int(sp[1]) & (2 ** 64 - 1), int(sp[2]) & (2 ** 64 - 1))
+    stride = int(sp[3]) if sp is not None and len(sp) > 3 else 0
     with torch.cuda.device(x.device):
-        rc = L.mvtb_kspace_chain_ex_f32(plan, _ptr(x), _ptr(y), nvol, host.desc_array(descs), len(descs), _ptr(pre_abt), _ptr(mm),
-                                        int(vols_per_sample), C.byref(spp) if spp is not None else None, _stream(x.device))
+        rc = L.mvtb_kspace_chain_ex_strided_f32(plan, _ptr(x), _ptr(y), nvol, host.desc_array(descs), len(descs), _ptr(pre_abt), _ptr(mm),
+                                                int(vols_per_sample), C.byref(spp) if spp is not None else None, C.c_uint64(stride),
+                                                _stream(x.device))
     _lib.check(L, rc)
     return (y, mm) if need_mm else y
 
