@@ -167,6 +167,28 @@ int mvtb_sparse_table(float p, unsigned* table_out);
 /* the uniforms mvtb_salt_pepper_f32 uses when u == NULL (for tests and for feeding the oracle) */
 int mvtb_philox_uniform_f32(float* out, size_t n, uint64_t seed, uint64_t offset, void* stream);
 
+/* ---- torch's CPU generator (MT19937) on the device, with host jump-ahead (csrc/mt19937.cuh).  torch.rand(n) in float32
+ * on the default CPU generator is the sequential MT19937 outputs y mapped to (y & 0xFFFFFF) 2^-24.  A state is torch's:
+ * the 624 words of torch.get_rng_state() (stored there as uint64) plus its `next` and `left`, which must be a state torch
+ * leaves: left = 1, or left = 625 - next with 1 <= next <= 624.  Polynomials are over GF(2) modulo the generator's
+ * characteristic polynomial phi (degree 19937), 19937 coefficients in 624 uint32, lowest first, in caller memory.
+ * mvtb_mt19937_jump_poly: poly_out = t^n mod phi.
+ * mvtb_mt19937_advance: moves (state, next, left) n draws ahead, as n draws of torch would.  For n >= 625 `poly` must be
+ *   mvtb_mt19937_jump_poly(n - 625) (the jump lands 624 words in front of the new position); below that it is unused.
+ * mvtb_mt19937_chunk_table: table_out[c] = t^(c chunk_len) mod phi for c < n_chunks (n_chunks x 624 uint32, host).
+ * mvtb_mt19937_uniform_f32: u[s][i] (device, n_segments x n) = what torch.rand(n) returns from state s.  states: device,
+ *   MVTB_MT_STATE_WORDS uint32 per segment (the 624 words, then next, then left).  table: the chunk table on the device;
+ *   one CTA per (segment, chunk of chunk_len) jumps there and runs the recurrence, n_chunks chunks per round, and a
+ *   segment longer than n_chunks chunks takes several rounds.  workspace: mvtb_mt19937_workspace_bytes(n_segments) of
+ *   device memory. */
+#define MVTB_MT_STATE_WORDS 640
+int mvtb_mt19937_jump_poly(uint64_t n, uint32_t* poly_out);
+int mvtb_mt19937_advance(const uint32_t* poly, uint64_t n, uint32_t* state, int32_t* next, int32_t* left);
+int mvtb_mt19937_chunk_table(uint64_t chunk_len, int n_chunks, uint32_t* table_out);
+size_t mvtb_mt19937_workspace_bytes(int n_segments);
+int mvtb_mt19937_uniform_f32(float* u, size_t n, int n_segments, const uint32_t* states, const uint32_t* table,
+                             uint64_t chunk_len, int n_chunks, void* workspace, void* stream);
+
 /* ---- intensity prologue: NormalizeIntensityd(nonzero=True, channel_wise=True) -> RandScaleIntensityd ->
  * RandShiftIntensityd, the MONAI 0.5 transforms in front of the chain in every training script of the reference
  * (10_scripts/127_.../stylized_gibbs12p5_spikes15_wrap0p5_sap0p05_FLAIR.py:134-136).  Per channel c with m = x != 0:

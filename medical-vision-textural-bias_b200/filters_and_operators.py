@@ -261,8 +261,10 @@ class RandPlaneWaves_ellipsoid(RandomizableTransform, MapTransform):
 class SaltAndPepper(MapTransform, RandomizableTransform):
     """Salt-and-pepper voxel corruption (F:419-482): u<=p/2 -> min/2, p/2<u<=p -> max/2.
 
-    rng="torch" (default) draws u with torch.rand on the CPU generator exactly where the reference does
-    (F:472), so seeded runs reproduce it bit for bit; rng="philox" draws u inside the kernel from
+    rng="torch" (default) draws u from torch's CPU generator exactly where the reference does (F:472), so seeded
+    runs reproduce it bit for bit: the stream is made on the device (mvtb_mt19937_uniform_f32) and the generator
+    advanced on the host by jump-ahead, with the same uniforms and the same generator state afterwards as
+    torch.rand(x.size()), which is still called when the default dtype is not float32; rng="philox" draws u inside the kernel from
     Philox4x32-10 keyed by `seed` (counter advances every call) and never touches host memory;
     rng="philox-sparse" walks from hit to hit with Philox-drawn geometric gaps (same Bernoulli(p) field
     statistics, cost proportional to p)."""
@@ -291,11 +293,17 @@ class SaltAndPepper(MapTransform, RandomizableTransform):
 
     def salt_and_pepper(self, x: torch.Tensor, u: Optional[torch.Tensor] = None):
         """x: any shape; min/max are taken over the whole tensor (F:476).  u: optional injected uniforms."""
-        if u is None and self.rng == "torch":
+        # torch.rand(x.size()) in float32 on the CPU generator is made on the device from the same stream (a float64
+        # default dtype draws doubles, and another default device another generator: those stay with torch.rand)
+        on_device = u is None and self.rng == "torch" and torch.get_default_dtype() == torch.float32 and \
+            torch.get_default_device().type == "cpu"
+        if u is None and self.rng == "torch" and not on_device:
             u = torch.rand(x.size())
         xd, src = Fn.to_device(x)
         ud = None
-        if u is not None:
+        if on_device:
+            ud = Fn.torch_uniform(xd.shape, 1, xd.device)[0]
+        elif u is not None:
             ud = u.to(device=xd.device, dtype=torch.float32).contiguous()
         sparse = ud is None and self.rng == "philox-sparse"
         y = Fn.salt_pepper(xd, float(self.p), u=ud, seed=self.seed, offset=self.offset, n_samples=1, sparse=sparse)

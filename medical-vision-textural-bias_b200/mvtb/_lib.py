@@ -91,6 +91,12 @@ _SYMBOLS = {
                                               C.c_void_p, C.c_void_p, C.c_void_p]),
     "mvtb_sparse_table": (C.c_int, [C.c_float, C.POINTER(C.c_uint32)]),
     "mvtb_philox_uniform_f32": (C.c_int, [C.c_void_p, C.c_size_t, C.c_uint64, C.c_uint64, C.c_void_p]),
+    "mvtb_mt19937_jump_poly": (C.c_int, [C.c_uint64, C.c_void_p]),
+    "mvtb_mt19937_advance": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
+    "mvtb_mt19937_chunk_table": (C.c_int, [C.c_uint64, C.c_int, C.c_void_p]),
+    "mvtb_mt19937_workspace_bytes": (C.c_size_t, [C.c_int]),
+    "mvtb_mt19937_uniform_f32": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int,
+                                           C.c_void_p, C.c_void_p]),
     "mvtb_intensity_scratch_bytes": (C.c_size_t, [C.c_int]),
     "mvtb_intensity_prologue_coeffs_f32": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                      C.c_void_p, C.c_void_p]),
@@ -120,6 +126,7 @@ _SYMBOLS = {
 }
 K_KINDS = 18
 SP_BLOCK = 256
+MT_STATE_WORDS = 640
 
 
 def bind(cdll):

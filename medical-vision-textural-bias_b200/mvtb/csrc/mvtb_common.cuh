@@ -18,6 +18,8 @@
 static inline float __double2float_rn(double d) { return (float)d; }
 static inline double __dmul_rn(double a, double b) { volatile double r = a * b; return r; }
 static inline double __dadd_rn(double a, double b) { volatile double r = a + b; return r; }
+// the jump's shared-memory reduction (mt19937.cuh); blocks run one thread at a time
+static inline unsigned atomicXor(unsigned* p, unsigned v) { unsigned o = *p; *p = o ^ v; return o; }
 #else
 #include <cuda_runtime.h>
 #define MVTB_LAUNCH(kern, grid, block, smem, stream, ...) \

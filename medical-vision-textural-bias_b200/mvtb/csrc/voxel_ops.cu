@@ -8,6 +8,7 @@
 #include "mvtb_common.cuh"
 #include "philox.cuh"
 #include "sp_sampler.cuh"
+#include "mt19937.cuh"
 
 namespace mvtb {
 

@@ -369,6 +369,131 @@ def philox_uniform(n: int, seed: int, offset: int, device: torch.device) -> torc
     return out
 
 
+# ----------------------------------------------------------------------------- torch's CPU generator on the device
+# torch.get_rng_state() of the default CPU generator: `left` (int32) at byte 8, `next` (uint64) at byte 16, then the 624
+# state words stored as uint64 (csrc/mt19937.cuh).
+_MT_N = 624
+_MT_LEFT, _MT_NEXT, _MT_WORDS = 8, 16, 24
+_mt_polys: "OrderedDict" = OrderedDict()
+_mt_tables: dict = {}
+_mt_lock = threading.Lock()
+
+
+def mt19937_unpack(state: torch.Tensor) -> Tuple[np.ndarray, int, int]:
+    """(words uint32[624], next, left) of a torch.get_rng_state() byte tensor."""
+    b = state.numpy() if isinstance(state, torch.Tensor) else np.asarray(state, dtype=np.uint8)
+    words = b[_MT_WORDS:_MT_WORDS + 8 * _MT_N].view(np.uint64).astype(np.uint32)
+    return words, int(b[_MT_NEXT:_MT_NEXT + 8].view(np.uint64)[0]), int(b[_MT_LEFT:_MT_LEFT + 4].view(np.int32)[0])
+
+
+def mt19937_pack(words: np.ndarray, next_: int, left: int, like: torch.Tensor) -> torch.Tensor:
+    """A copy of the byte tensor `like` (a torch.get_rng_state()) carrying this generator state."""
+    out = like.clone()
+    b = out.numpy()
+    b[_MT_WORDS:_MT_WORDS + 8 * _MT_N].view(np.uint64)[:] = np.asarray(words, dtype=np.uint32)
+    b[_MT_NEXT:_MT_NEXT + 8].view(np.uint64)[0] = next_
+    b[_MT_LEFT:_MT_LEFT + 4].view(np.int32)[0] = left
+    return out
+
+
+def _mt_poly(n: int) -> np.ndarray:
+    """The jump polynomial mvtb_mt19937_advance needs for n >= 625 draws (a few per process: one per distinct n)."""
+    with _mt_lock:
+        p = _mt_polys.get(n)
+        if p is not None:
+            _mt_polys.move_to_end(n)
+            return p
+    L = _lib.lib()
+    p = np.empty(_MT_N, dtype=np.uint32)
+    _lib.check(L, L.mvtb_mt19937_jump_poly(C.c_uint64(n - 625), C.c_void_p(p.ctypes.data)))
+    with _mt_lock:
+        _mt_polys[n] = p
+        while len(_mt_polys) > 64:
+            _mt_polys.popitem(last=False)
+    return p
+
+
+def mt19937_advance(words: np.ndarray, next_: int, left: int, n: int) -> Tuple[np.ndarray, int, int]:
+    """The generator state n draws later, as torch would leave it (host jump-ahead; `words` is updated in place)."""
+    L = _lib.lib()
+    words = np.ascontiguousarray(words, dtype=np.uint32)
+    nx, lf = C.c_int32(next_), C.c_int32(left)
+    poly = _mt_poly(n) if n >= 625 else None
+    _lib.check(L, L.mvtb_mt19937_advance(None if poly is None else C.c_void_p(poly.ctypes.data), C.c_uint64(n),
+                                         C.c_void_p(words.ctypes.data), C.byref(nx), C.byref(lf)))
+    return words, nx.value, lf.value
+
+
+def mt19937_take(n: int, segments: int, out: Optional[np.ndarray] = None) -> np.ndarray:
+    """Consume segments x n draws of the default CPU generator on the host: returns each segment's start state as rows of
+    _lib.MT_STATE_WORDS int32 (words, next, left; `out` if given) and leaves the generator where segments calls of
+    torch.rand(n) would.  Touches no CUDA state."""
+    st = torch.get_rng_state()
+    words, nx, lf = mt19937_unpack(st)
+    rows = np.zeros((segments, _lib.MT_STATE_WORDS), dtype=np.int32) if out is None else out
+    for s in range(segments):
+        rows[s, :_MT_N] = words.view(np.int32)
+        rows[s, _MT_N], rows[s, _MT_N + 1] = nx, lf
+        words, nx, lf = mt19937_advance(words, nx, lf, n)
+    torch.set_rng_state(mt19937_pack(words, nx, lf, st))
+    return rows
+
+
+def _mt_geometry(n: int, segments: int) -> Tuple[int, int]:
+    # at most one CTA per SM, in one round: the jump costs each CTA the same whatever its chunk's length, so fewer, longer
+    # chunks win until the SMs run out.  Powers of two keep the number of distinct tables small.
+    # (measured on a B200: a second round, or a second CTA on an SM, costs more than longer chunks do)
+    n_chunks = 128
+    per_seg = max(1, min(n_chunks, 148 // segments))
+    chunk = max(1024, 1 << max(0, (-(-n // per_seg) - 1).bit_length()))
+    return chunk, n_chunks
+
+
+def _mt_table(dev: torch.device, chunk: int, n_chunks: int) -> torch.Tensor:
+    key = (dev.index, chunk, n_chunks)
+    t = _mt_tables.get(key)
+    if t is None:
+        L = _lib.lib()
+        h = np.empty((n_chunks, _MT_N), dtype=np.uint32)
+        _lib.check(L, L.mvtb_mt19937_chunk_table(C.c_uint64(chunk), n_chunks, C.c_void_p(h.ctypes.data)))
+        t = torch.from_numpy(h.view(np.int32)).to(dev)
+        _mt_tables[key] = t
+    return t
+
+
+def mt19937_uniform(states: torch.Tensor, n: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """u[s] = what torch.rand(n) returns from start state s, float32 (segments, n) on states' device.  states: a CUDA int32
+    (segments, MT_STATE_WORDS) tensor of mt19937_take rows."""
+    L = _lib.lib()
+    S = int(states.shape[0])
+    if not states.is_cuda or states.dtype != torch.int32 or tuple(states.shape) != (S, _lib.MT_STATE_WORDS) or not states.is_contiguous():
+        raise ValueError(f"states must be a contiguous int32 CUDA tensor of shape (segments, {_lib.MT_STATE_WORDS})")
+    dev = states.device
+    u = torch.empty((S, n), dtype=torch.float32, device=dev) if out is None else out
+    if n == 0 or S == 0:
+        return u
+    chunk, n_chunks = _mt_geometry(n, S)
+    table = _mt_table(dev, chunk, n_chunks)
+    ws = torch.empty(int(L.mvtb_mt19937_workspace_bytes(S)), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        rc = L.mvtb_mt19937_uniform_f32(_ptr(u), n, S, _ptr(states), _ptr(table), C.c_uint64(chunk), n_chunks, _ptr(ws), _stream(dev))
+    _lib.check(L, rc)
+    return u
+
+
+def torch_uniform(shape, segments: int = 1, device: Optional[torch.device] = None) -> torch.Tensor:
+    """`segments` consecutive torch.rand(shape) draws of the default CPU generator, made on the device: a float32 CUDA
+    tensor (segments, *shape) equal bit for bit to them, and the generator left where they would leave it.  The state is
+    advanced on the host by jump-ahead; the host is never synchronised with the device."""
+    require_cuda()
+    shape = (int(shape),) if isinstance(shape, (int, np.integer)) else tuple(int(s) for s in shape)
+    n = math.prod(shape)
+    dev = device or torch.device("cuda", torch.cuda.current_device())
+    pinned = torch.empty((segments, _lib.MT_STATE_WORDS), dtype=torch.int32, pin_memory=True)
+    mt19937_take(n, segments, out=pinned.numpy())
+    return mt19937_uniform(pinned.to(dev, non_blocking=True), n).view((segments,) + shape)
+
+
 def wrap_fold(x: torch.Tensor, alpha: float) -> torch.Tensor:
     """Even-axis wraparound fold on (..., H, W, D); raises MvtbError(EUNSUPPORTED) for an odd axis."""
     L = _lib.lib()

@@ -140,7 +140,7 @@ class TrainStage:
         mvtb.intensity.NormalizeIntensityd(nonzero=True, channel_wise=True) -> RandScaleIntensityd -> RandShiftIntensityd,
             or IntensityPrologued (scale / shift need the normalisation in front of them)
         filters_and_operators.RandFourierDiskMaskd(inside_off=False) -> RandPlaneWaves_ellipsoid -> WrapArtifactd
-            -> SaltAndPepper(prob=1, rng="philox" or "philox-sparse")
+            -> SaltAndPepper(prob=1, rng="philox" or "philox-sparse"; rng="torch" with torch_generator=True)
 
     with filters_and_operators.SelectChanneld anywhere and MONAI's ToTensord as a no-op.  The intensity and k-space
     transforms act on one key (the image).  A SelectChanneld in front of the salt-and-pepper is folded into the gather;
@@ -154,12 +154,21 @@ class TrainStage:
     per-worker reseeding (worker_init_fn) changes the draws, as it does for the reference.  The copies include the
     salt-and-pepper `offset`, which starts equal in every worker and never advances in the main process: give each worker
     its own `sp.seed` in worker_init_fn (records carry the seed they were drawn with), or the workers' salt-and-pepper
-    patterns repeat."""
+    patterns repeat.
 
-    def __init__(self, cache: DeviceCache, transforms: Sequence):
+    SaltAndPepper(rng="torch") draws its uniforms from torch's process-wide CPU generator, as the reference does; a stage
+    takes it only with `torch_generator=True`, since consuming that generator is a side effect.  Per-sample torch.rand calls
+    consume the stream one after another, so `draw` records the generator's state at its first sample (the others continue
+    that stream) and advances the generator on the host by jump-ahead, once, by what all its samples' torch.rand would take:
+    a batch leaves it where per-sample calls would.  `apply` makes the uniforms on the device from the recorded states
+    (mvtb_mt19937_uniform_f32) and selects with them.  In forked DataLoader workers each worker's generator is seeded by
+    torch per worker, as for the reference."""
+
+    def __init__(self, cache: DeviceCache, transforms: Sequence, torch_generator: bool = False):
         F = _ops()
         self.cache = cache
         self.tail = list(transforms)
+        self.torch_generator = bool(torch_generator)
         cached = set(cache.keys)
         ch = {k: list(range(cache.channels[k])) for k in cache.keys}     # current channel map per key (into the cache)
         self.pre_select = None                          # channel maps at the salt-and-pepper (what the gather reads)
@@ -223,8 +232,9 @@ class TrainStage:
             elif n == "WrapArtifactd":
                 self.wrap = t
             else:
-                if t.rng not in ("philox", "philox-sparse"):
-                    raise NotImplementedError(f"TrainStage: SaltAndPepper(rng={t.rng!r}) draws on the host; use rng='philox' "
+                if t.rng not in ("philox", "philox-sparse") and not (t.rng == "torch" and self.torch_generator):
+                    raise NotImplementedError(f"TrainStage: SaltAndPepper(rng={t.rng!r}) draws from torch's global generator; "
+                                              "pass torch_generator=True to let the stage consume it, or use rng='philox' "
                                               "or 'philox-sparse'")
                 if t.prob != 1:
                     raise NotImplementedError("TrainStage: SaltAndPepper needs prob=1")
@@ -261,8 +271,9 @@ class TrainStage:
         """Every random parameter of the batch `indices`, sample after sample, from the transforms' own randomize (and the
         salt-and-pepper offsets, which advance as per-sample calls advance them).  Touches no CUDA state."""
         rec = {k: [] for k in ("index", "start", "size", "flip", "scale_gate", "factor", "shift_gate", "offset", "disk_gate",
-                               "r", "spike_gate", "spike_idx", "sp_gate", "sp_seed", "sp_offset", "sp_blocks")}
+                               "r", "spike_gate", "spike_idx", "sp_gate", "sp_seed", "sp_offset", "sp_blocks", "sp_state")}
         first = self.crop.keys[0] if self.crop is not None else self.cache.keys[0]
+        mt = None                                       # rng="torch": the generator at the draw's start, and the draws taken
         for i in indices:
             i = int(i)
             rec["index"].append(i)
@@ -298,12 +309,23 @@ class TrainStage:
                 elif t is self.sp:
                     t.randomize(None)
                     n = len(self.pre_select[self.image_key]) * math.prod(size)
+                    if t.rng == "torch":                # prob=1: every sample draws torch.rand(n)
+                        if torch.get_default_dtype() != torch.float32:
+                            raise RuntimeError("TrainStage: SaltAndPepper(rng='torch') draws float32 uniforms; torch.rand "
+                                               f"would draw {torch.get_default_dtype()} under this default dtype")
+                        # the samples' streams follow each other: the first records its start state, the others continue it
+                        if mt is None:
+                            mt = [Fn.mt19937_take(0, 1)[0], 0]
+                            rec["sp_state"].append(mt[0])
+                        else:
+                            rec["sp_state"].append(None)
+                        mt[1] += n
                     blocks = (n + 255) // 256 if t.rng == "philox-sparse" else (n + 3) // 4
                     rec["sp_gate"].append(bool(t._do_transform))
                     rec["sp_seed"].append(int(t.seed))
                     rec["sp_offset"].append(int(t.offset))
                     rec["sp_blocks"].append(blocks)
-                    if t._do_transform:
+                    if t._do_transform and t.rng != "torch":
                         t.offset += blocks
             if self.scale is not None:
                 rec["scale_gate"].append(bool(self.scale._do_transform))
@@ -314,6 +336,10 @@ class TrainStage:
             rec["start"].append(start)
             rec["size"].append(size)
             rec["flip"].append(fm)
+        if mt is not None:                              # one host jump for the whole draw
+            st = torch.get_rng_state()
+            words, nx, lf = Fn.mt19937_advance(mt[0][:624].view(np.uint32).copy(), int(mt[0][624]), int(mt[0][625]), mt[1])
+            torch.set_rng_state(Fn.mt19937_pack(words, nx, lf, st))
         return rec
 
     def __len__(self) -> int:
@@ -367,7 +393,10 @@ class TrainStage:
         # the per-sample arrays of every step, uploaded in one copy from pinned memory
         n_int = 5 * B
         n_flt = 2 * B * c_img if has_int else 0
-        pinned = torch.empty(n_int + n_flt, dtype=torch.int32, pin_memory=True)
+        torch_sp = self.sp is not None and self.sp.rng == "torch"
+        runs = [b for b in range(B) if rec["sp_state"][b] is not None] if torch_sp else []
+        n_mt = len(runs) * _lib.MT_STATE_WORDS
+        pinned = torch.empty(n_int + n_flt + n_mt, dtype=torch.int32, pin_memory=True)
         pv = pinned.numpy()
         pv[:B] = idx
         pv[B:4 * B] = starts.reshape(-1)
@@ -377,9 +406,11 @@ class TrainStage:
                 np.where(rec["scale_gate"], 1.0 + np.asarray(rec["factor"], dtype=np.float64), 1.0).astype(np.float32)
             sh = np.zeros(B, dtype=np.float32) if self.shift is None else \
                 np.where(rec["shift_gate"], np.asarray(rec["offset"], dtype=np.float64), 0.0).astype(np.float32)
-            fv = pv[n_int:].view(np.float32)
+            fv = pv[n_int:n_int + n_flt].view(np.float32)
             fv[:B * c_img] = np.repeat(sc, c_img)
             fv[B * c_img:] = np.repeat(sh, c_img)
+        if torch_sp:
+            pv[n_int + n_flt:] = np.stack([rec["sp_state"][b] for b in runs]).reshape(-1)
         up = pinned.to(dev, non_blocking=True)
         entry_d, starts_d, flips_d = up[:B], up[B:4 * B], up[4 * B:5 * B]
         L = _lib.lib()
@@ -399,10 +430,11 @@ class TrainStage:
             abt = None
             if has_int:
                 scale_d = up[n_int:n_int + B * c_img].view(torch.float32)
-                shift_d = up[n_int + B * c_img:].view(torch.float32)
+                shift_d = up[n_int + B * c_img:n_int + n_flt].view(torch.float32)
                 abt = Fn.intensity_coeffs(x, B * c_img, scale=scale_d, shift=shift_d)
             if self.disk or self.wave or self.wrap or self.sp:
-                x = self._chain(x, rec, roi, B, c_img, abt)
+                states = (runs, up[n_int + n_flt:].view(len(runs), _lib.MT_STATE_WORDS)) if torch_sp else None
+                x = self._chain(x, rec, roi, B, c_img, abt, states)
             elif abt is not None:
                 x = Fn.intensity_affine(x, abt, out=x)
             out[ik] = x
@@ -412,7 +444,7 @@ class TrainStage:
             out[mk] = [cache.meta[i][mk] for i in rec["index"]]
         return out
 
-    def _chain(self, x, rec, roi, B, c_img, abt):
+    def _chain(self, x, rec, roi, B, c_img, abt, states=None):
         descs = []
         for b in range(B):
             r = rec["r"][b] if self.disk is not None and rec["disk_gate"][b] else None
@@ -427,6 +459,19 @@ class TrainStage:
         contiguous = all(rec["sp_gate"]) and all(off[b] == off[0] + b * blocks[0] and blocks[b] == blocks[0] and seed[b] == seed[0]
                                                  for b in range(B))
         sparse = sp.rng == "philox-sparse"
+        if states is not None:                          # rng="torch": the uniforms of every sample's torch.rand
+            y, mm = Fn.kspace_chain_ex(x, 3, descs, pre_abt=abt, want_minmax=True, vols_per_sample=c_img, out=x)
+            starts, st = states                         # sample starts[j] .. starts[j + 1] - 1 continue one stream
+            n = y[0].numel()
+            bounds = starts + [B]
+            lens = {bounds[j + 1] - bounds[j] for j in range(len(starts))}
+            u = torch.empty_like(y)
+            if len(lens) == 1:                          # runs of equal length: one call, a segment per run
+                Fn.mt19937_uniform(st, lens.pop() * n, out=u.view(len(starts), -1))
+            else:
+                for j in range(len(starts)):
+                    Fn.mt19937_uniform(st[j:j + 1], (bounds[j + 1] - bounds[j]) * n, out=u[bounds[j]:bounds[j + 1]].view(1, -1))
+            return Fn.salt_pepper(y, float(sp.p), u=u, n_samples=B, mm=mm, out=y)
         if sparse and contiguous:
             return Fn.kspace_chain_ex(x, 3, descs, pre_abt=abt, sp=(float(sp.p), seed[0], off[0], blocks[0]), vols_per_sample=c_img,
                                       out=x)[0]
@@ -443,6 +488,9 @@ class TrainStage:
         """apply(draw(batch)) for the batches of BatchSampler(RandomSampler / SequentialSampler): the order of a DataLoader
         with the same arguments and generator."""
         src = range(len(self.cache))
+        if self.torch_generator:
+            # a DataLoader draws its base seed before the sampler's: the generator then ends an epoch where one leaves it
+            torch.empty((), dtype=torch.int64).random_(generator=generator)
         sampler = RandomSampler(src, generator=generator) if shuffle else SequentialSampler(src)
         for batch in BatchSampler(sampler, batch_size, drop_last):
             yield self.apply(self.draw(batch))
