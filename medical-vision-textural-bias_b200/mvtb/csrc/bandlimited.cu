@@ -779,12 +779,14 @@ static void is_build_pattern(int A, int B, int lag, int spread, std::vector<unsi
     *max_back = mb;
 }
 
-// shared memory of the fused W/D kernel: the [K][K] bins share the front of the buffer with the W table
+// shared memory of the fused W/D kernel: the [K][K] bins share the front of the buffer with the W table; then the
+// [K][D] W-bins (later [K][F + 1] float4, which needs K + 1 columns when D = K) and the [D] twiddles
 template <int NF>
 static size_t bl_midw_smem(const BlGeom& g, int K) {
     const size_t smem_w = sizeof(float) * (size_t)(g.W / 2 + 1) * BlDims<NF>::NT;
     const size_t bins = sizeof(cf) * (size_t)K * K;
-    return ((smem_w > bins ? smem_w : bins) + 15) / 16 * 16 + sizeof(cf) * ((size_t)K * g.D + g.D);
+    const size_t cols = g.D > K ? (size_t)g.D : (size_t)K + 1;
+    return ((smem_w > bins ? smem_w : bins) + 15) / 16 * 16 + sizeof(cf) * ((size_t)K * cols + g.D);
 }
 
 template <int NF>

@@ -615,7 +615,8 @@ k_bl_midw(cf* __restrict__ Y, BlGeom g, const BlVol* __restrict__ vols, int vol_
     float* sc = (float*)smem_raw;                        // (cos, sin) rows of the W axis, 0 .. W/2
     cf* sb = (cf*)smem_raw;                              // [K][K]  bins after the pointwise stage
     cf* sg = (cf*)(smem_raw + front);                    // [K][D]  W-bins of every column
-    cf* st = sg + K * D;                                 // [D]     exp(-2 pi i t / D)
+    // the way back reuses sg as [K][F + 1] float4 = K (K + 1) cf, one row more than [K][D] holds when D = K
+    cf* st = sg + (size_t)K * (D > K ? D : K + 1);       // [D]     exp(-2 pi i t / D)
     const int tid = threadIdx.x, nthr = blockDim.x;
     const int vol = blockIdx.x / NF, fh = blockIdx.x - vol * NF;
     bl_load_table<NF>(sc, g.tabC[1], g.tabS[1], W, tid, nthr);

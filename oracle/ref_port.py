@@ -253,7 +253,9 @@ def chain_127_exact_phase(x: torch.Tensor, r: float, idx, intensity: float, alph
     injected amplitude equal."""
     xd = x.to(torch.float64)
     k = kspace(xd, 3)
-    k = k * disk_binary_mask(k.shape, r, 3, False).to(torch.float64)
+    m = disk_binary_mask(k.shape, r, 3, False).to(torch.float64)
+    # +0 in the masked bins: 0 * k is -0 where Re k < 0, and angle(-0 + 0j) = pi would flip the spike's sign
+    k = torch.where(m > 0, k * m, torch.zeros_like(k))
     # the reference goes back to the image and forward again between stages; in exact arithmetic that is the identity
     la = k.abs().log()
     ph = k.angle()                                       # angle(0) = 0 for the exactly-zero masked bins
