@@ -75,7 +75,8 @@ class ConvertToMultiChannelBasedOnBratsClassesd(MapTransform):
 
 
 class WholeTumorTCGA(MapTransform):
-    """TCGA segmentation -> whole-tumour mask with a channel axis (F:90-101)."""
+    """TCGA segmentation -> whole-tumour mask with a channel axis (F:90-101).  A CUDA tensor (mvtb.nifti.LoadImaged's output)
+    stays on its device and comes back as CUDA float32."""
 
     def __init__(self, keys, allow_missing_keys=False):
         MapTransform.__init__(self, keys, allow_missing_keys)
@@ -83,6 +84,10 @@ class WholeTumorTCGA(MapTransform):
     def __call__(self, data):
         d = dict(data)
         for key in self.key_iterator(d):
+            lab = d[key]
+            if isinstance(lab, torch.Tensor) and lab.is_cuda:
+                d[key] = (lab != 0)[None].to(torch.float32)
+                continue
             d[key] = (d[key] != 0)[None, :].astype(np.float32)
         return d
 

@@ -12,7 +12,8 @@ flip, as in MONAI (the window is drawn from the first key's shape).
 
 In front of them, `Spacingd` -> `Orientationd` (127_...FLAIR.py:120-129) resample the loaded volume to the training grid:
 `resample` runs both, plus an optional window and flip, as one gather (`mvtb_resample_f32`, csrc/resample.cuh) on the
-geometry of mvtb/geometry.py; `SpacingOrientationd` is the two drop-ins in one pass."""
+geometry of mvtb/geometry.py; `SpacingOrientationd` is the two drop-ins in one pass, and each drop-in's `resample_crop` takes
+a `CenterSpatialCropd` that follows it into the same gather (the validation prefix, 127_...FLAIR.py:153)."""
 import ctypes as C
 import threading
 from collections import OrderedDict
@@ -307,12 +308,22 @@ class _Resampled(MapTransform):
         self.meta_key_postfix = meta_key_postfix
 
     def __call__(self, data):
+        return self.resample_crop(data)
+
+    def resample_crop(self, data, crop: Optional["CenterSpatialCropd"] = None):
+        """__call__ followed by `crop` (a CenterSpatialCropd on some of this transform's keys), the crop fused into the
+        gather of each key it acts on: one read of the loaded volume and one write of the crop.  The same bits and the
+        same meta dicts as the two transforms in sequence (the crop leaves the affine alone)."""
+        if crop is not None and not set(crop.keys) <= set(self.keys):
+            raise ValueError(f"resample_crop: the crop's keys {list(crop.keys)} are not all among {list(self.keys)}")
         d = dict(data)
+        cropped = set(crop.key_iterator(d)) if crop is not None else set()
         for key, mode, pm, ac, dt in self.key_iterator(d, self.mode, self.padding_mode, self.align_corners, self.dtype):
             meta = d[f"{key}_{self.meta_key_postfix}"]
             p = Geo.plan(meta["affine"], tuple(d[key].shape[1:]), self.pixdim, self.diagonal, self.axcodes,
                          self.as_closest_canonical, self.labels)
-            d[key] = resample(d[key], p, mode, padding_mode=pm, align_corners=ac, dtype=dt)
+            window = center_window(p.shape, crop.roi_size) if key in cropped else None
+            d[key] = resample(d[key], p, mode, window=window, padding_mode=pm, align_corners=ac, dtype=dt)
             meta["affine"] = p.affine
         return d
 

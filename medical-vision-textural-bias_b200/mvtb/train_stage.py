@@ -4,7 +4,8 @@ random tail of the Compose applied to a whole batch.
 
     DeviceCache(data, prefix)      runs the deterministic prefix (LoadImaged -> AsChannelFirstd -> ConvertToMultiChannel ->
                                    Spacingd / Orientationd, ...) once per item, on threads, and keeps every key of every item
-                                   in one flat float32 device buffer per key (what MONAI's CacheDataset holds, on the GPU)
+                                   in one flat float32 device buffer per key (what MONAI's CacheDataset holds, on the GPU);
+                                   for validation the prefix ends in CenterSpatialCropd, fused into the resampling gather
     TrainStage(cache, transforms)  the random tail (RandSpatialCropd -> RandFlipd -> intensity prologue -> disk -> plane wave
                                    -> wrap -> salt-and-pepper, each optional, SelectChanneld anywhere) as a handful of launches
                                    per batch: one crop + flip gather per key (mvtb_crop_flip_gather_f32), one statistics pass,
@@ -46,10 +47,42 @@ def _keys(t) -> List[str]:
 
 # ----------------------------------------------------------------------------------------------------------------- cache
 
+class ResampleCenterCrop:
+    """A Spacingd / Orientationd / SpacingOrientationd and the CenterSpatialCropd right behind it, on some of its keys, as one
+    step of a cache fill: each cropped key is one windowed gather (mvtb.spatial's resample_crop)."""
+
+    def __init__(self, resample, crop):
+        self.resample, self.crop = resample, crop
+
+    def __call__(self, data):
+        return self.resample.resample_crop(data, self.crop)
+
+
+def fill_steps(prefix: Sequence) -> list:
+    """The steps a DeviceCache runs for `prefix`: the transforms themselves, except that a CenterSpatialCropd directly behind
+    a resampling transform, acting on a subset of its keys, joins it as one ResampleCenterCrop."""
+    steps: list = []
+    for t in prefix:
+        prev = steps[-1] if steps else None
+        if (isinstance(t, S.CenterSpatialCropd) and isinstance(prev, (S.Spacingd, S.Orientationd, S.SpacingOrientationd))
+                and set(_keys(t)) <= set(_keys(prev))):
+            steps[-1] = ResampleCenterCrop(prev, t)
+        else:
+            steps.append(t)
+    return steps
+
+
 class DeviceCache:
     """Every item of `data` (the scripts' list of dicts, e.g. {"image": path, "label": path}) after the deterministic
     `prefix`, on the device.  Allowed in the prefix: mvtb.nifti.LoadImaged / AsChannelFirstd, filters_and_operators'
-    ConvertToMultiChannelBasedOnBratsClassesd / SelectChanneld, mvtb.spatial.Spacingd / Orientationd / SpacingOrientationd.
+    ConvertToMultiChannelBasedOnBratsClassesd / WholeTumorTCGA / SelectChanneld, mvtb.spatial.Spacingd / Orientationd /
+    SpacingOrientationd / CenterSpatialCropd.
+
+    A CenterSpatialCropd directly behind Spacingd, Orientationd or SpacingOrientationd, on a subset of its keys (the
+    validation prefix), is fused into the resampling gather of those keys (`fill_steps`): the fill then reads the loaded
+    volume once and writes only the crop, with the same bits and meta dicts as the two transforms in sequence.  Anywhere
+    else it runs as the drop-in.  As in MONAI, a volume smaller than the roi on some axis gives a smaller crop; the cache
+    holds it like any other ragged entry, and TrainStage.apply refuses a batch of different sizes with ValueError.
 
     The prefix runs per item on `num_workers` threads (the loaders and the resampling are thread-safe).  Each array key
     (a (C, H, W, D) volume; C equal for all items, H, W, D free, as Spacingd makes them) then lives in one flat float32
@@ -59,15 +92,15 @@ class DeviceCache:
 
     def __init__(self, data: Sequence[dict], prefix: Sequence, num_workers: int = 4, device: Optional[torch.device] = None):
         F = _ops()
-        allowed = (N.LoadImaged, N.AsChannelFirstd, F.ConvertToMultiChannelBasedOnBratsClassesd, F.SelectChanneld,
-                   S.Spacingd, S.Orientationd, S.SpacingOrientationd)
+        allowed = (N.LoadImaged, N.AsChannelFirstd, F.ConvertToMultiChannelBasedOnBratsClassesd, F.WholeTumorTCGA,
+                   F.SelectChanneld, S.Spacingd, S.Orientationd, S.SpacingOrientationd, S.CenterSpatialCropd)
         for t in prefix:
             if not isinstance(t, allowed):
                 raise NotImplementedError(f"DeviceCache: {_name(t)} is not a supported prefix transform "
                                           f"(supported: {', '.join(a.__name__ for a in allowed)})")
         Fn.require_cuda()
         self.device = device or torch.device("cuda", torch.cuda.current_device())
-        prefix = list(prefix)
+        prefix = fill_steps(prefix)
 
         def one(item):
             d = dict(item)
@@ -145,6 +178,11 @@ class TrainStage:
     with filters_and_operators.SelectChanneld anywhere and MONAI's ToTensord as a no-op.  The intensity and k-space
     transforms act on one key (the image).  A SelectChanneld in front of the salt-and-pepper is folded into the gather;
     one behind it (the select takes its min / max over all channels) is applied to the result.
+
+    Without a RandSpatialCropd the stage gathers whole entries, so every sample of a batch needs the same cached shape
+    (ValueError otherwise).  On a cache whose prefix ends in CenterSpatialCropd this is the scripts' validation tail
+    (SelectChanneld -> NormalizeIntensityd -> disk -> plane wave -> wrap -> salt-and-pepper), and loader(batch_size,
+    shuffle=False) visits the samples in the validation DataLoader's order.
 
     `draw(indices)` (host only) returns a record of every random parameter; `apply(record)` returns the batch as CUDA
     float32 tensors (B, C, *roi) per key, plus per-sample lists of the meta dicts.  `loader(...)` yields
