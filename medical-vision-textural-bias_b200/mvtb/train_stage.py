@@ -22,6 +22,7 @@ when the stage is built."""
 import ctypes as C
 import math
 import types
+from collections.abc import Sequence as _SeqABC
 from concurrent.futures import ThreadPoolExecutor
 from typing import Dict, List, Optional, Sequence
 
@@ -162,7 +163,9 @@ class DeviceCache:
 # position of each supported transform in the 127 scripts' order; SelectChanneld and ToTensord may sit anywhere
 _RANK = {"RandSpatialCropd": 0, "RandFlipd": 1, "NormalizeIntensityd": 2, "RandScaleIntensityd": 3, "RandShiftIntensityd": 4,
          "IntensityPrologued": (2, 4), "RandFourierDiskMaskd": 5, "RandPlaneWaves_ellipsoid": 6, "WrapArtifactd": 7,
-         "SaltAndPepper": 8}
+         "SaltAndPepper": 8, "RandGibbsNoised": 5, "RandKSpaceSpikeNoised": 6}
+# the augmentation transforms, accepted with kspace_augment=True; each takes the slot of the one it cannot share a tail with
+_AUGMENT = {"RandGibbsNoised": "RandFourierDiskMaskd", "RandKSpaceSpikeNoised": "RandPlaneWaves_ellipsoid"}
 
 
 class TrainStage:
@@ -200,20 +203,43 @@ class TrainStage:
     that stream) and advances the generator on the host by jump-ahead, once, by what all its samples' torch.rand would take:
     a batch leaves it where per-sample calls would.  `apply` makes the uniforms on the device from the recorded states
     (mvtb_mt19937_uniform_f32) and selects with them.  In forked DataLoader workers each worker's generator is seeded by
-    torch per worker, as for the reference."""
+    torch per worker, as for the reference.
 
-    def __init__(self, cache: DeviceCache, transforms: Sequence, torch_generator: bool = False):
+    `kspace_augment=True` also accepts the k-space augmentation of the 20_Gibbs_filters and 30_augmentation scripts, on
+    the image key:
+
+        filters_and_operators.RandGibbsNoised(as_tensor_output=True)       in the disk's slot (1 to 8 channels)
+        filters_and_operators.RandKSpaceSpikeNoised(intensity_ranges={image: ...}, as_tensor_output=True)
+                                                                            in the plane wave's slot; channel_wise and
+                                                                            common_sampling either way
+
+    Without the keyword both are refused, as before.  The Gibbs transform cannot share a tail with the disk, nor the spikes
+    with the plane wave (a chain descriptor holds one mask and one spike source); the spikes need a given intensity range
+    (the default one is computed from the image's spectrum, which `draw` cannot see), and no SelectChanneld on the image
+    between them and the salt-and-pepper (their draws are per channel).  `draw` calls the objects' own `_randomize`
+    sample after sample: the Gibbs gate and alpha, the spikes' global gate, the common_sampling reseed and the inner
+    per-channel gates, locations and intensities, on a shape-only stand-in of the (C, *roi) image.  `apply` builds one
+    chain descriptor per channel volume and runs the k-space chain only on the samples with something to do (a gate on,
+    or a WrapArtifactd in the tail): those are compacted, chained with their intensity map, and put back; the others
+    get the intensity map alone and are what the per-sample drop-ins leave, bit for bit.  The salt-and-pepper then
+    runs over the whole batch with the counters per-sample calls use."""
+
+    def __init__(self, cache: DeviceCache, transforms: Sequence, torch_generator: bool = False, kspace_augment: bool = False):
         F = _ops()
         self.cache = cache
         self.tail = list(transforms)
         self.torch_generator = bool(torch_generator)
+        self.kspace_augment = bool(kspace_augment)
         cached = set(cache.keys)
         ch = {k: list(range(cache.channels[k])) for k in cache.keys}     # current channel map per key (into the cache)
         self.pre_select = None                          # channel maps at the salt-and-pepper (what the gather reads)
         self.post_select: Dict[str, List[int]] = {}     # channels of the result kept after the salt-and-pepper
         self.crop = self.flip = self.norm = self.scale = self.shift = self.disk = self.wave = self.wrap = self.sp = None
+        self.gibbs = self.kspike = None
+        kspike_ch = None                                # the image's channel map where the spikes are drawn
         self.image_key = None
         last = -1
+        seen = set()
         for t in self.tail:
             n = _name(t)
             if n == "ToTensord":
@@ -226,8 +252,17 @@ class TrainStage:
                          "IntensityPrologued": I.IntensityPrologued, "RandFourierDiskMaskd": F.RandFourierDiskMaskd,
                          "RandPlaneWaves_ellipsoid": F.RandPlaneWaves_ellipsoid, "WrapArtifactd": F.WrapArtifactd,
                          "SaltAndPepper": F.SaltAndPepper}
+            if self.kspace_augment:
+                supported.update(RandGibbsNoised=F.RandGibbsNoised, RandKSpaceSpikeNoised=F.RandKSpaceSpikeNoised)
+            elif n in _AUGMENT:
+                raise NotImplementedError(f"TrainStage: {n} is not supported; pass kspace_augment=True to run it in the stage")
             if n not in supported or not isinstance(t, supported[n]):
                 raise NotImplementedError(f"TrainStage: {n} is not supported")
+            for a, b in _AUGMENT.items():
+                if (n == a and b in seen) or (n == b and a in seen):
+                    raise NotImplementedError(f"TrainStage: {a} and {b} in one tail; a chain descriptor holds one "
+                                              + ("mask" if a == "RandGibbsNoised" else "spike source"))
+            seen.add(n)
             lo, hi = _RANK[n] if isinstance(_RANK[n], tuple) else (_RANK[n], _RANK[n])
             if lo <= last:
                 raise NotImplementedError(f"TrainStage: {n} after a transform that comes later in the 127 scripts' order "
@@ -269,6 +304,22 @@ class TrainStage:
                 self.wave = t
             elif n == "WrapArtifactd":
                 self.wrap = t
+            elif n == "RandGibbsNoised":
+                if not t.as_tensor_output:
+                    raise NotImplementedError("TrainStage: RandGibbsNoised(as_tensor_output=False) returns numpy arrays")
+                self.gibbs = t
+            elif n == "RandKSpaceSpikeNoised":
+                inner = t.transforms[keys[0]]
+                if not t.as_tensor_output:
+                    raise NotImplementedError("TrainStage: RandKSpaceSpikeNoised(as_tensor_output=False) returns numpy arrays")
+                if inner.intensity_range is None:
+                    raise NotImplementedError("TrainStage: RandKSpaceSpikeNoised without intensity_ranges for the image key; the "
+                                              "default range comes from the image's spectrum, which draw() cannot see")
+                rng = inner.intensity_range
+                if isinstance(rng[0], _SeqABC) and len(rng) != len(ch[keys[0]]):
+                    raise ValueError(f"TrainStage: RandKSpaceSpikeNoised has {len(rng)} intensity ranges for an image of "
+                                     f"{len(ch[keys[0]])} channels; one per channel is needed")
+                self.kspike, kspike_ch = t, list(ch[keys[0]])
             else:
                 if t.rng not in ("philox", "philox-sparse") and not (t.rng == "torch" and self.torch_generator):
                     raise NotImplementedError(f"TrainStage: SaltAndPepper(rng={t.rng!r}) draws from torch's global generator; "
@@ -288,6 +339,9 @@ class TrainStage:
                 raise NotImplementedError(f"TrainStage: {len(v)} channels of {k!r} in the gather; at most 8")
         if self.image_key is None:
             self.image_key = cache.keys[0]
+        if self.kspike is not None and kspike_ch != self.pre_select[self.image_key]:
+            raise NotImplementedError("TrainStage: a SelectChanneld on the image between RandKSpaceSpikeNoised and the "
+                                      "salt-and-pepper (or the end); the spikes are drawn per channel of the image they see")
         self._descs: dict = {}
 
     def _select(self, t, ch, cached):
@@ -310,6 +364,10 @@ class TrainStage:
         salt-and-pepper offsets, which advance as per-sample calls advance them).  Touches no CUDA state."""
         rec = {k: [] for k in ("index", "start", "size", "flip", "scale_gate", "factor", "shift_gate", "offset", "disk_gate",
                                "r", "spike_gate", "spike_idx", "sp_gate", "sp_seed", "sp_offset", "sp_blocks", "sp_state")}
+        if self.gibbs is not None:
+            rec.update(gibbs_gate=[], alpha=[])
+        if self.kspike is not None:
+            rec.update(kspike_gate=[], kspikes=[])
         first = self.crop.keys[0] if self.crop is not None else self.cache.keys[0]
         mt = None                                       # rng="torch": the generator at the draw's start, and the draws taken
         for i in indices:
@@ -344,6 +402,14 @@ class TrainStage:
                         idx = tuple(int(v) for v in t.idx)
                     rec["spike_gate"].append(bool(t._do_transform))
                     rec["spike_idx"].append(idx)
+                elif t is self.gibbs:
+                    t._randomize(None)                  # the gate, then alpha, which is always drawn
+                    rec["gibbs_gate"].append(bool(t._do_transform))
+                    rec["alpha"].append(float(t.sampled_alpha))
+                elif t is self.kspike:
+                    gate, spikes = self._draw_kspikes(t, size)
+                    rec["kspike_gate"].append(gate)
+                    rec["kspikes"].append(spikes)
                 elif t is self.sp:
                     t.randomize(None)
                     n = len(self.pre_select[self.image_key]) * math.prod(size)
@@ -380,6 +446,25 @@ class TrainStage:
             torch.set_rng_state(Fn.mt19937_pack(words, nx, lf, st))
         return rec
 
+    def _draw_kspikes(self, t, size):
+        """RandKSpaceSpikeNoised's draws for one sample, as its __call__ makes them: the global gate, the common_sampling
+        reseed, then the inner transform's per-channel draws on a (C, *size) stand-in of the image (shape only, no memory).
+        Returns the gate and, when it is on, one (fftshift-ed (x, y, z), log-intensity) or None per channel."""
+        t.randomize(None)
+        if t.common_sampling:
+            for k in t.keys:
+                t.transforms[k].set_random_state(t.common_seed)
+        if not t._do_transform:
+            return False, None
+        inner = t.transforms[self.image_key]
+        img = np.broadcast_to(np.zeros((), np.uint8), (len(self.pre_select[self.image_key]),) + tuple(size))
+        inner.sampled_k_intensity, inner.sampled_locs = [], []
+        inner._randomize(img, inner._make_sequence(img))
+        spikes = [None] * img.shape[0]
+        for loc, v in zip(inner.sampled_locs, inner.sampled_k_intensity):
+            spikes[loc[0]] = (tuple(int(i) for i in loc[1:]), float(v))
+        return True, tuple(spikes)
+
     def __len__(self) -> int:
         return len(self.cache)
 
@@ -387,15 +472,18 @@ class TrainStage:
         return self.draw([i])
 
     # ---- device side
-    def _desc(self, roi, r, idx):
-        key = (roi, r, idx)
+    def _desc(self, roi, mask, spikes):
+        """mask: None, ("disk", r) or ("gibbs", alpha); spikes: ((fftshift-ed (x, y, z), log-intensity), ...)"""
+        key = (roi, mask, spikes)
         d = self._descs.get(key)
         if d is None:
             kw = {}
-            if r is not None:
-                kw.update(mask_kind=_lib.MASK_DISK, mask_ndim=3, mask_thresh=host.disk_threshold(r, roi))
-            if idx is not None:
-                kw["spikes"] = [(idx, host.exp_f32(self.wave.intensity_value))]
+            if mask is not None and mask[0] == "disk":
+                kw.update(mask_kind=_lib.MASK_DISK, mask_ndim=3, mask_thresh=host.disk_threshold(mask[1], roi))
+            elif mask is not None:
+                kw.update(mask_kind=_lib.MASK_CENTRED, mask_ndim=3, mask_thresh=host.gibbs_threshold(mask[1], roi))
+            if spikes:
+                kw["spikes"] = [(idx, host.exp_f32(v)) for idx, v in spikes]
             if self.wrap is not None:
                 kw["wrap_alpha"] = float(self.wrap.transform.alpha)
             d = host.make_desc(**kw)
@@ -403,6 +491,21 @@ class TrainStage:
                 self._descs.clear()
             self._descs[key] = d
         return d
+
+    def _sample_descs(self, rec, b, roi, c_img):
+        """The chain descriptors of sample b, one per channel volume, and whether the chain has anything to do on it"""
+        mask = None
+        if self.disk is not None and rec["disk_gate"][b]:
+            mask = ("disk", rec["r"][b])
+        elif self.gibbs is not None and rec["gibbs_gate"][b]:
+            mask = ("gibbs", rec["alpha"][b])
+        spikes = [()] * c_img
+        if self.wave is not None and rec["spike_idx"][b] is not None:
+            spikes = [((rec["spike_idx"][b], self.wave.intensity_value),)] * c_img
+        elif self.kspike is not None and rec["kspikes"][b] is not None:
+            spikes = [() if s is None else (s,) for s in rec["kspikes"][b]]
+        busy = mask is not None or any(spikes) or self.wrap is not None
+        return [self._desc(roi, mask, s) for s in spikes], busy
 
     def apply(self, record) -> dict:
         """The batch of `record` (a draw, or a list of draws) on the device: {key: (B, C, *roi) float32 CUDA tensor,
@@ -434,7 +537,14 @@ class TrainStage:
         torch_sp = self.sp is not None and self.sp.rng == "torch"
         runs = [b for b in range(B) if rec["sp_state"][b] is not None] if torch_sp else []
         n_mt = len(runs) * _lib.MT_STATE_WORDS
-        pinned = torch.empty(n_int + n_flt + n_mt, dtype=torch.int32, pin_memory=True)
+        descs, gated = None, None                       # kspace_augment: the samples the chain runs on, when not all
+        if self.gibbs is not None or self.kspike is not None:
+            per = [self._sample_descs(rec, b, roi, c_img) for b in range(B)]
+            descs = [d for ds, busy in per if busy for d in ds]
+            if not all(busy for _, busy in per):
+                gated = [b for b in range(B) if per[b][1]]
+        o_g = n_int + n_flt + n_mt + (n_int + n_flt + n_mt) % 2        # int64 indices at an 8-byte boundary
+        pinned = torch.empty(o_g + 2 * len(gated) if gated else n_int + n_flt + n_mt, dtype=torch.int32, pin_memory=True)
         pv = pinned.numpy()
         pv[:B] = idx
         pv[B:4 * B] = starts.reshape(-1)
@@ -448,7 +558,9 @@ class TrainStage:
             fv[:B * c_img] = np.repeat(sc, c_img)
             fv[B * c_img:] = np.repeat(sh, c_img)
         if torch_sp:
-            pv[n_int + n_flt:] = np.stack([rec["sp_state"][b] for b in runs]).reshape(-1)
+            pv[n_int + n_flt:n_int + n_flt + n_mt] = np.stack([rec["sp_state"][b] for b in runs]).reshape(-1)
+        if gated:
+            pv[o_g:].view(np.int64)[:] = gated
         up = pinned.to(dev, non_blocking=True)
         entry_d, starts_d, flips_d = up[:B], up[B:4 * B], up[4 * B:5 * B]
         L = _lib.lib()
@@ -470,9 +582,12 @@ class TrainStage:
                 scale_d = up[n_int:n_int + B * c_img].view(torch.float32)
                 shift_d = up[n_int + B * c_img:n_int + n_flt].view(torch.float32)
                 abt = Fn.intensity_coeffs(x, B * c_img, scale=scale_d, shift=shift_d)
-            if self.disk or self.wave or self.wrap or self.sp:
-                states = (runs, up[n_int + n_flt:].view(len(runs), _lib.MT_STATE_WORDS)) if torch_sp else None
-                x = self._chain(x, rec, roi, B, c_img, abt, states)
+            if self.disk or self.wave or self.wrap or self.sp or self.gibbs is not None or self.kspike is not None:
+                states = (runs, up[n_int + n_flt:n_int + n_flt + n_mt].view(len(runs), _lib.MT_STATE_WORDS)) if torch_sp else None
+                if gated is None:
+                    x = self._chain(x, rec, roi, B, c_img, abt, states, descs)
+                else:
+                    x = self._chain_gated(x, rec, B, c_img, abt, states, descs, up[o_g:].view(torch.int64) if gated else None)
             elif abt is not None:
                 x = Fn.intensity_affine(x, abt, out=x)
             out[ik] = x
@@ -482,23 +597,50 @@ class TrainStage:
             out[mk] = [cache.meta[i][mk] for i in rec["index"]]
         return out
 
-    def _chain(self, x, rec, roi, B, c_img, abt, states=None):
-        descs = []
-        for b in range(B):
-            r = rec["r"][b] if self.disk is not None and rec["disk_gate"][b] else None
-            idx = rec["spike_idx"][b] if self.wave is not None else None
-            descs.extend([self._desc(roi, r, idx)] * c_img)
+    def _chain(self, x, rec, roi, B, c_img, abt, states=None, descs=None):
+        if descs is None:
+            descs = [d for b in range(B) for d in self._sample_descs(rec, b, roi, c_img)[0]]
         descs = host.desc_array(descs)
         sp = self.sp
         if sp is None or not any(rec["sp_gate"]):
             return Fn.kspace_chain_ex(x, 3, descs, pre_abt=abt, out=x)
+        if states is None and sp.rng == "philox-sparse" and self._sp_contiguous(rec, B):
+            off, blocks, seed = rec["sp_offset"], rec["sp_blocks"], rec["sp_seed"]
+            return Fn.kspace_chain_ex(x, 3, descs, pre_abt=abt, sp=(float(sp.p), seed[0], off[0], blocks[0]), vols_per_sample=c_img,
+                                      out=x)[0]
+        y, mm = Fn.kspace_chain_ex(x, 3, descs, pre_abt=abt, want_minmax=True, vols_per_sample=c_img, out=x)
+        return self._salt_pepper(y, mm, rec, B, states)
+
+    def _chain_gated(self, x, rec, B, c_img, abt, states, descs, g):
+        """The k-space chain on the samples `g` (int64 indices on the device; None: no sample) alone: compacted, chained with
+        their slice of the intensity map, put back.  The others get the intensity map alone, as the per-sample drop-ins
+        pass them through without an FFT.  The salt-and-pepper then runs over the whole batch."""
+        if g is not None:
+            xg = x.index_select(0, g)
+            abt_g = None if abt is None else abt.view(B, c_img, 3).index_select(0, g).view(-1, 3)
+        if abt is not None:
+            Fn.intensity_affine(x, abt, out=x)
+        if g is not None:
+            x.index_copy_(0, g, Fn.kspace_chain_ex(xg, 3, host.desc_array(descs), pre_abt=abt_g, out=xg))
+        if self.sp is None or not any(rec["sp_gate"]):
+            return x
+        return self._salt_pepper(x, Fn.minmax(x, B), rec, B, states)
+
+    @staticmethod
+    def _sp_contiguous(rec, B):
+        """do the batch's salt-and-pepper counters follow each other as per-sample calls would have used them?"""
+        off, blocks, seed = rec["sp_offset"], rec["sp_blocks"], rec["sp_seed"]
+        return all(rec["sp_gate"]) and all(off[b] == off[0] + b * blocks[0] and blocks[b] == blocks[0] and seed[b] == seed[0]
+                                           for b in range(B))
+
+    def _salt_pepper(self, y, mm, rec, B, states=None):
+        """The select on the batch y (min / max per sample in mm) with the recorded counters or torch states"""
+        sp = self.sp
         off, blocks, seed = rec["sp_offset"], rec["sp_blocks"], rec["sp_seed"]
         # one select call when the batch's counters follow each other as per-sample calls would have used them
-        contiguous = all(rec["sp_gate"]) and all(off[b] == off[0] + b * blocks[0] and blocks[b] == blocks[0] and seed[b] == seed[0]
-                                                 for b in range(B))
+        contiguous = self._sp_contiguous(rec, B)
         sparse = sp.rng == "philox-sparse"
         if states is not None:                          # rng="torch": the uniforms of every sample's torch.rand
-            y, mm = Fn.kspace_chain_ex(x, 3, descs, pre_abt=abt, want_minmax=True, vols_per_sample=c_img, out=x)
             starts, st = states                         # sample starts[j] .. starts[j + 1] - 1 continue one stream
             n = y[0].numel()
             bounds = starts + [B]
@@ -510,10 +652,8 @@ class TrainStage:
                 for j in range(len(starts)):
                     Fn.mt19937_uniform(st[j:j + 1], (bounds[j + 1] - bounds[j]) * n, out=u[bounds[j]:bounds[j + 1]].view(1, -1))
             return Fn.salt_pepper(y, float(sp.p), u=u, n_samples=B, mm=mm, out=y)
-        if sparse and contiguous:
-            return Fn.kspace_chain_ex(x, 3, descs, pre_abt=abt, sp=(float(sp.p), seed[0], off[0], blocks[0]), vols_per_sample=c_img,
-                                      out=x)[0]
-        y, mm = Fn.kspace_chain_ex(x, 3, descs, pre_abt=abt, want_minmax=True, vols_per_sample=c_img, out=x)
+        # philox-sparse: the standalone select numbers a batch's spans per sample, not by the offsets per-sample calls use, so
+        # it runs sample by sample (the stride that fixes that is only in the chain's fused select)
         n = y[0].numel()
         if not sparse and contiguous and n % 4 == 0:      # dense Philox: element i of the batch uses counter offset + i / 4
             return Fn.salt_pepper(y, float(sp.p), seed=seed[0], offset=off[0], n_samples=B, mm=mm, out=y)
